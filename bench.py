@@ -58,7 +58,29 @@ def parse():
     ap.add_argument("--merge", default="p2p", choices=["p2p", "nccl"],
                     help="N>1 ensemble-merge: p2p = votes stored into every rank's buffer from the kernel epilogue over "
                          "NVLink peer memory (fused); nccl = a separate all_gather per step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed (rank 0) as DIR/<name>.npy, float32 or "
+                         "float64, at most 64 MB in all (a fixed seeded sample of rows when larger): the same arguments give "
+                         "the same inputs, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the device path: --impl b200")
+    return args
+
+
+DUMP_BYTES = 60 << 20  # of array data: the .npy headers stay within 64 MB beside it
+
+
+def dump_rows(n, bytes_per_row):
+    """the rows a dump keeps: all n when they fit DUMP_BYTES, else a fixed seeded sample of them (sorted)"""
+    k = DUMP_BYTES // bytes_per_row
+    return np.arange(n) if n <= k else np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+
+
+def dump_arrays(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------ workloads
@@ -709,6 +731,12 @@ def main():
         oks = [None] * world
         dist.all_gather_object(oks, merge_check)
         merge_check = all(oks)
+    if args.dump_outputs and rank == 0:
+        # the last launch read rotating buffer k, the base batch shifted down by k * 977 rows: shifting its scores back puts
+        # them in the base batch's row order whichever buffer that was (`inner`, hence k, is sized from a timing probe)
+        scores = mine if merge == "p2p" else out.cpu().numpy().reshape(B, plan.out_cols)
+        scores = np.roll(scores, -((inner * args.steps - 1) % nbuf) * 977, axis=0)
+        dump_arrays(args.dump_outputs, {"outputs": scores[dump_rows(B, scores.itemsize * plan.out_cols)]})
 
     # kernel-only time of the dominant kernel (no collective), for the roofline
     n_k = max(args.steps * inner, 10)
@@ -848,7 +876,7 @@ def main():
             import copy
 
             sub = copy.copy(args)
-            sub.no_cpu_baseline, sub.steps, sub.warmup, sub.batch = True, 200, 3, 0
+            sub.no_cpu_baseline, sub.steps, sub.warmup, sub.batch, sub.dump_outputs = True, 200, 3, 0, None
             for nm, fn in (("ingest6", main_ingest), ("enrich_ens4", main_enrich)):
                 try:
                     row = compact_line(fn(sub, 0, local_rank, 1, emit=False))
@@ -951,6 +979,19 @@ def main_ingest(args, rank, local_rank, world, emit=True):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        # every result column of the last step, as the slots hold it: float32 columns as they are, integer columns as
+        # float64, timestamps as float64 seconds since the epoch
+        specs, _extra = iplan._landing()
+        rows = torch.from_numpy(dump_rows(B, 8 * len(specs))).cuda()
+        cols = {}
+        for col, slot, dt in specs:
+            tdt = {np.float32: torch.float32, np.int32: torch.int32, np.int64: torch.int64}[dt.type]
+            a = out[slot * stride: slot * stride + B * dt.itemsize].view(tdt)[rows].cpu().numpy()
+            if dt == np.int64:
+                a = (a // 10**9).astype(np.float64) + (a % 10**9) * 1e-9
+            cols[col] = a if dt == np.float32 else a.astype(np.float64)
+        dump_arrays(args.dump_outputs, cols)
     n_it = max(args.steps, 10)
     kms = plan.time_device([b.data_ptr() for b in bufs], stride, B, out.data_ptr(), stride, cnt.data_ptr(), n_it) / n_it
     lat = []
@@ -1166,6 +1207,9 @@ def main_enrich(args, rank, local_rank, world, emit=True):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        scores = out.cpu().numpy().reshape(B, plan.out_cols)
+        dump_arrays(args.dump_outputs, {"outputs": scores[dump_rows(B, scores.itemsize * plan.out_cols)]})
     n_it = max(args.steps, 10)
     lat = []
     if fused:  # the step IS the kernel: time it alone, and one 4096-key launch for the latency figure

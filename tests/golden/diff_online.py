@@ -1,11 +1,12 @@
 """The checker of the enrichment path -- oracle/enrichment.py's OnlineVectorService restatement -- against the REAL
-OnlineVectorService (feature_store/feature_vector.py:903-1067; build container only; the online-store read is the same dict
-stub under both, as in the `online_service_logic` scenario): random tables (floats, ints, nan, +-inf, None, missing features,
-all-zero rows), random impute policies ("*" and per-feature constants and $mean / $min / $max / $std / $count statistics, unknown
-and label features), with and without label column / index columns, single and composite keys; lookups as lists, dicts, a
-single dict, unknown keys, extra columns, malformed asks.  Results, impute tables and exceptions compared.
+OnlineVectorService (feature_store/feature_vector.py:903-1067; the online-store read is the same dict stub under both, as in
+the `online_service_logic` scenario): random tables (floats, ints, nan, +-inf, None, missing features, all-zero rows), random
+impute policies ("*" and per-feature constants and $mean / $min / $max / $std / $count statistics, unknown and label features),
+with and without label column / index columns, single and composite keys; lookups as lists, dicts, a single dict, unknown keys,
+extra columns, malformed asks.  Results, impute tables and exceptions compared.  The reference's answers are stored in
+tests/golden/reference_checks.json.xz (gen_reference_checks.py), so the CPU suite runs `check` against them on any machine.
 
-    python -m tests.golden.diff_online
+    python -m tests.golden.diff_online      (live, needs the reference)
 """
 import os
 import random
@@ -15,8 +16,9 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspa
 import pandas as pd  # noqa: E402
 
 from tests import api_oracle as ora  # noqa: E402
-from tests.golden import api_reference as ref  # noqa: E402
 from tests.scenarios import _first_line  # noqa: E402
+
+VERDICT = "identical on 500 random online services"
 
 
 def norm(v):
@@ -38,10 +40,10 @@ def attempt(fn):
         return {"raised": type(exc).__name__, "message": _first_line(str(exc))}
 
 
-def main():
+def services():
+    """the 500 seeded cases: (feats, index, table, stats, label, with_idx, policy, composite, asks)"""
     rnd = random.Random(23)
-    n = 0
-    for case in range(500):
+    for _case in range(500):
         nf = rnd.randint(1, 6)
         feats = [f"f{i}" for i in range(nf)]
         label = rnd.choice([None, feats[-1]]) if nf > 1 else None
@@ -69,27 +71,50 @@ def main():
         with_idx = rnd.random() < 0.3
         keys = list(table) + [("nobody", 9) if composite else ("nobody",)]
         asks = [list(rnd.choice(keys)) for _ in range(rnd.randint(1, 4))]
-        out = []
-        for api in (ref, ora):
-            def go(api=api):
-                svc = api.online_service(feats, index, table, stats, label, with_idx, policy)
-                res = {"impute": norm(dict(svc._impute_values)),
-                       "lists": attempt(lambda: svc.get(asks, as_list=True)),
-                       "dicts": attempt(lambda: svc.get([dict(zip(index, a)) for a in asks])),
-                       "one": attempt(lambda: svc.get(dict(zip(index, asks[0])))),
-                       "extra": attempt(lambda: svc.get([{**dict(zip(index, asks[0])), "note": 1}])),
-                       "short": attempt(lambda: svc.get([asks[0][:1]])) if composite else None,
-                       "empty": attempt(lambda: svc.get([])), "string": attempt(lambda: svc.get("k0"))}
-                return res
-            out.append(repr(attempt(go)))
-        n += 1
-        if out[0] != out[1]:
+        yield feats, index, table, stats, label, with_idx, policy, composite, asks
+
+
+def answers(api):
+    """repr of everything `api`'s OnlineVectorService answers, per case"""
+    out = []
+    for feats, index, table, stats, label, with_idx, policy, composite, asks in services():
+        def go():
+            svc = api.online_service(feats, index, table, stats, label, with_idx, policy)
+            res = {"impute": norm(dict(svc._impute_values)),
+                   "lists": attempt(lambda: svc.get(asks, as_list=True)),
+                   "dicts": attempt(lambda: svc.get([dict(zip(index, a)) for a in asks])),
+                   "one": attempt(lambda: svc.get(dict(zip(index, asks[0])))),
+                   "extra": attempt(lambda: svc.get([{**dict(zip(index, asks[0])), "note": 1}])),
+                   "short": attempt(lambda: svc.get([asks[0][:1]])) if composite else None,
+                   "empty": attempt(lambda: svc.get([])), "string": attempt(lambda: svc.get("k0"))}
+            return res
+        out.append(repr(attempt(go)))
+    return out
+
+
+def reference_answers():
+    from tests.golden import api_reference as ref
+
+    return answers(ref)
+
+
+def check(reference):
+    """the oracle against `reference` (what reference_answers returned)"""
+    mine = answers(ora)
+    assert len(mine) == len(reference)
+    for case, (want, got, args) in enumerate(zip(reference, mine, services())):
+        if want != got:
+            feats, index, table, _stats, label, with_idx, policy, _composite, asks = args
             print("DIFF", case, feats, label, index, table, policy, with_idx, asks)
-            print("  ref :", out[0][:1200])
-            print("  mine:", out[1][:1200])
+            print("  ref :", want[:1200])
+            print("  mine:", got[:1200])
             return 1
-    print("identical on", n, "random online services")
+    print(VERDICT)
     return 0
+
+
+def main():
+    return check(reference_answers())
 
 
 if __name__ == "__main__":
