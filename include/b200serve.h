@@ -318,6 +318,48 @@ int b2s_cols_run_host(b2s_cols_t plan, const void* const* h_in_slots, int64_t n_
 int b2s_cols_time_device(b2s_cols_t plan, const void* const* d_in, int32_t n_bufs, int64_t in_slot_stride, int64_t n_rows,
                          void* d_out, int64_t out_slot_stride, uint64_t* d_counters, int32_t n_iters, float* total_ms);
 
+/* ---- feature-set statistics: ingest(..., infer_options=Stats | Histogram) on the device -------------------------------
+ * get_df_stats (data_types/infer.py:104-149), called on the ingested frame by _infer_from_static_df
+ * (feature_store/api.py:1162-1196): pandas describe(include="all") plus a 20-bin np.histogram per column.  The columns of a
+ * plan's result are described where they are: the plan's resident result of its last b2s_cols_run_host (d_out NULL), or a
+ * caller's device buffer in the b2s_cols_run_device layout.  Two calls, because the host needs the first summary to choose
+ * what the second pass computes (histogram edges from min / max, target ranks from the count):
+ *   begin   one pass: per column count, missing, fp64 sum, min, max, +-inf, ones (bool), row 0 -> summary[n_cols];
+ *   finish  the centred sum of squares around means[i] (NaN: none), the 20 histogram counts with the host's edges, and up to
+ *           B2S_STAT_RANKS exact order statistics per column (radix select over the same data; ranks[i][r] < 0: none).
+ * Stats kinds say how a slot is read and what is missing.  The calls run on the library stream and block until their results
+ * are on the host.  A b2s_cols_run_host of the plan between begin and finish replaces the result: finish then fails with
+ * B2S_ERR_STATE (call begin again). */
+#define B2S_STAT_F32 0      /* float32 slot; NaN is missing                                   */
+#define B2S_STAT_I32 1      /* int32 slot                                                     */
+#define B2S_STAT_I32_NAT 2  /* int32 date part; -1 marks NaT (missing)                        */
+#define B2S_STAT_BOOL 3     /* int32 0 / 1 slot                                               */
+#define B2S_STAT_DT 4       /* int64 nanoseconds over two slots; NaT (INT64_MIN) is missing   */
+#define B2S_STAT_ROW 5      /* the row number (no slot is read)                               */
+#define B2S_STAT_RANKS 6
+#define B2S_STAT_BINS 20
+typedef struct b2s_colsum {
+  int64_t count;          /* non-missing values                                                         */
+  int64_t missing;
+  int64_t ones;           /* B2S_STAT_BOOL: values equal to 1                                            */
+  int32_t pos_inf, neg_inf;
+  double sum;             /* fp64, added in a fixed order                                               */
+  int64_t min_bits;       /* min / max of the non-missing values: float32 bits for B2S_STAT_F32, else the */
+  int64_t max_bits;       /*   integer value (count > 0 only)                                           */
+  int64_t first_bits;     /* row 0, in the same encoding                                                */
+  int32_t first_missing;
+  int32_t pad_;
+} b2s_colsum;
+int b2s_cols_stats_begin(b2s_cols_t plan, const void* d_out, int64_t out_slot_stride, int64_t n_rows, const int32_t* kinds,
+                         const int32_t* slots, int32_t n_cols, b2s_colsum* summary, b2s_stats* stats);
+/* hist_kind[i]: 0 none, 1 float32 bins, 2 float64 bins (np.histogram's bin dtype); hist[i] = 23 doubles: first_edge,
+ * last_edge - first_edge, then the 21 edges, all exact values of the bin dtype.  Outputs: m2[n_cols],
+ * hist_counts[n_cols][B2S_STAT_BINS], order_values[n_cols][B2S_STAT_RANKS] (the encoding of b2s_colsum.min_bits). */
+int b2s_cols_stats_finish(b2s_cols_t plan, const double* means, const int32_t* hist_kind, const double* hist,
+                          const int64_t* ranks, double* m2, int64_t* hist_counts, int64_t* order_values, b2s_stats* stats);
+/* CUDA-event time and bytes read of each pass of the last begin / finish pair (pass 0 is begin's), kernel launches */
+int b2s_cols_stats_timing(b2s_cols_t plan, float* pass_ms, int64_t* pass_bytes, int32_t* n_passes, int32_t* launches);
+
 /* ---- body codec (host code): the step on either side of the path for HTTP / stream triggers ------------
  * GraphServer.run json-decodes the request body (serving/server.py:262-277) and _process_response json.dumps
  * the result (:298-308).  b2s_json_parse_inputs finds the top-level "inputs" member of a V2 body and converts

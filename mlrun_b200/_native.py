@@ -24,6 +24,8 @@ ROW_NONFINITE_INPUT, ROW_BAD_LABEL, ROW_UNKNOWN_KEY = 1, 2, 4
 CMP_LE, CMP_LT = 0, 1          # left when x <= threshold (scikit-learn, LightGBM) | x < threshold (xgboost)
 NAN_ERROR, NAN_DEFAULT_CHILD = 0, 1
 COL_F32, COL_I32, COL_I64 = 0, 1, 2
+STAT_F32, STAT_I32, STAT_I32_NAT, STAT_BOOL, STAT_DT, STAT_ROW = 0, 1, 2, 3, 4, 5
+STAT_RANKS, STAT_BINS = 6, 20
 DATE_PARTS = {"year": 0, "month": 1, "day": 2, "hour": 3, "minute": 4, "second": 5, "day_of_week": 6, "dayofweek": 6,
               "weekday": 6, "day_of_year": 7, "dayofyear": 7, "quarter": 8, "is_leap_year": 9, "days_in_month": 10,
               "daysinmonth": 10, "is_month_start": 11, "is_month_end": 12, "is_quarter_start": 13, "is_quarter_end": 14,
@@ -41,6 +43,13 @@ class Stats(C.Structure):
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class ColSum(C.Structure):
+    """b2s_colsum: pass 0 of the feature-set statistics, one per described column"""
+    _fields_ = [("count", C.c_int64), ("missing", C.c_int64), ("ones", C.c_int64), ("pos_inf", C.c_int32),
+                ("neg_inf", C.c_int32), ("sum", C.c_double), ("min_bits", C.c_int64), ("max_bits", C.c_int64),
+                ("first_bits", C.c_int64), ("first_missing", C.c_int32), ("pad_", C.c_int32)]
 
 
 class DevInfo(C.Structure):
@@ -118,6 +127,10 @@ SIGNATURES = {
     "b2s_cols_info": (C.c_int, [_vp, _pi32, _pi32]),
     "b2s_cols_run_device": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _vp, _vp]),
     "b2s_cols_run_host": (C.c_int, [_vp, C.POINTER(_vp), _i64, C.POINTER(_vp), C.POINTER(_u64), C.POINTER(Stats)]),
+    "b2s_cols_stats_begin": (C.c_int, [_vp, _vp, _i64, _i64, _pi32, _pi32, _i32, _vp, C.POINTER(Stats)]),
+    "b2s_cols_stats_finish": (C.c_int, [_vp, _pf64, _pi32, _pf64, C.POINTER(_i64), _pf64, C.POINTER(_i64), C.POINTER(_i64),
+                                        C.POINTER(Stats)]),
+    "b2s_cols_stats_timing": (C.c_int, [_vp, _pf32, C.POINTER(_i64), _pi32, _pi32]),
     # online feature table
     "b2s_table_create": (C.c_int, [C.POINTER(_i64), _i64, _pf32, _i32, _pf32, C.POINTER(_vp)]),
     "b2s_table_destroy": (C.c_int, [_vp]),

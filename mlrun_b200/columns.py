@@ -121,6 +121,44 @@ class ColumnsPlan:
                                                  int(out_stride), d_counters, int(iters), C.byref(ms)))
         return ms.value
 
+    # ---- feature-set statistics over the result (b2s_cols_stats_*): see feature_store/infer.py
+    def stats_begin(self, kinds, slots, n_rows, d_out=None, out_stride=0):
+        """pass 0 over the result columns `slots` (read as `kinds`, nat.STAT_*) of the last run_host (or of d_out):
+        a structured array of nat.ColSum records, one per column, and the call's timing"""
+        kinds = np.ascontiguousarray(kinds, dtype=np.int32)
+        slots = np.ascontiguousarray(slots, dtype=np.int32)
+        summary = (nat.ColSum * len(kinds))()
+        stats = nat.Stats()
+        nat.check(self._lib.b2s_cols_stats_begin(self._h, d_out, int(out_stride), int(n_rows), nat._p(kinds, C.c_int32),
+                                                 nat._p(slots, C.c_int32), len(kinds), summary, C.byref(stats)))
+        return np.ctypeslib.as_array(summary).copy(), stats.as_dict()
+
+    def stats_finish(self, means, hist_kind, hist, ranks):
+        """the passes after stats_begin: (sum of squares around means, histogram counts, order statistics), timing"""
+        n = len(means)
+        means = np.ascontiguousarray(means, dtype=np.float64)
+        hist_kind = np.ascontiguousarray(hist_kind, dtype=np.int32)
+        hist = np.ascontiguousarray(hist, dtype=np.float64).reshape(n, 23)
+        ranks = np.ascontiguousarray(ranks, dtype=np.int64).reshape(n, nat.STAT_RANKS)
+        m2 = np.zeros(n, dtype=np.float64)
+        counts = np.zeros((n, nat.STAT_BINS), dtype=np.int64)
+        order = np.zeros((n, nat.STAT_RANKS), dtype=np.int64)
+        stats = nat.Stats()
+        i64 = C.POINTER(C.c_int64)
+        nat.check(self._lib.b2s_cols_stats_finish(self._h, nat._p(means, C.c_double), nat._p(hist_kind, C.c_int32),
+                                                  nat._p(hist, C.c_double), nat._p(ranks, C.c_int64), nat._p(m2, C.c_double),
+                                                  counts.ctypes.data_as(i64), order.ctypes.data_as(i64), C.byref(stats)))
+        return m2, counts, order, stats.as_dict()
+
+    def stats_timing(self):
+        """per pass of the last begin / finish pair: CUDA-event ms and bytes read; and the kernel launches"""
+        ms = np.zeros(6, dtype=np.float32)
+        nbytes = np.zeros(6, dtype=np.int64)
+        n, launches = C.c_int32(), C.c_int32()
+        nat.check(self._lib.b2s_cols_stats_timing(self._h, nat._p(ms, C.c_float), nbytes.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                  C.byref(n), C.byref(launches)))
+        return {"pass_ms": ms[: n.value].tolist(), "pass_bytes": nbytes[: n.value].tolist(), "launches": launches.value}
+
     def close(self):
         if self._h:
             self._lib.b2s_cols_destroy(self._h)

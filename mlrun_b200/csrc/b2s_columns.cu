@@ -40,6 +40,9 @@ struct b2s_cols_s {
   char *d_in = nullptr, *d_out = nullptr;
   unsigned long long* d_cnt = nullptr;
   int64_t cap_rows = 0;
+  int64_t res_rows = 0, res_stride = 0;  // what d_out holds after the last host run (b2s_cols_stats_begin reads it there)
+  unsigned long long res_gen = 0;        // host runs so far (the statistics calls check that the result is still theirs)
+  ColStatsWS* stats_ws = nullptr;
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   std::vector<cudaEvent_t> chunk_ev;  // one per row range of a pipelined host run
 };
@@ -315,6 +318,8 @@ extern "C" int b2s_cols_run_host(b2s_cols_t c, const void* const* h_in_slots, in
     std::lock_guard<std::mutex> lk(c->mu);
     COL_TRY(cudaSetDevice(b2s_int_device()));
     const int64_t stride = ((n_rows * 4 + 255) / 256) * 256;
+    c->res_rows = 0;
+    ++c->res_gen;
     const size_t n_out = c->out_words.size();
     if (n_rows > c->cap_rows) {
       if (c->d_in) { cudaFree(c->d_in); cudaFree(c->d_out); c->d_in = c->d_out = nullptr; }
@@ -402,6 +407,8 @@ extern "C" int b2s_cols_run_host(b2s_cols_t c, const void* const* h_in_slots, in
       COL_TRY(cudaEventRecord(c->ev[3], st));
       COL_TRY(cudaStreamSynchronize(st));
       COL_TRY(cudaStreamSynchronize(cs));
+      c->res_rows = n_rows;
+      c->res_stride = stride;
       if (stats) {
         memset(stats, 0, sizeof(*stats));
         stats->rows = n_rows;
@@ -428,6 +435,8 @@ extern "C" int b2s_cols_run_host(b2s_cols_t c, const void* const* h_in_slots, in
     if (c->n_counters) COL_TRY(cudaMemcpyAsync(counters, c->d_cnt, c->n_counters * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     COL_TRY(cudaEventRecord(c->ev[3], st));
     COL_TRY(cudaStreamSynchronize(st));
+    c->res_rows = n_rows;
+    c->res_stride = stride;
     if (stats) {
       memset(stats, 0, sizeof(*stats));
       stats->rows = n_rows;
@@ -442,6 +451,22 @@ extern "C" int b2s_cols_run_host(b2s_cols_t c, const void* const* h_in_slots, in
   }
 }
 
+std::mutex& b2s_int_cols_mutex(b2s_cols_s* c) { return c->mu; }
+
+int b2s_int_cols_result(b2s_cols_s* c, const char** d_out, long long* stride, long long* rows, int* n_out_slots,
+                        unsigned long long* generation) {
+  if (!c || !c->finalized) return b2s_int_fail(B2S_ERR_STATE, "plan not finalized");
+  *generation = c->res_gen;
+  if (!c->res_rows) return b2s_int_fail(B2S_ERR_STATE, "the plan holds no result: run it with b2s_cols_run_host first (or pass d_out)");
+  *d_out = c->d_out;
+  *stride = c->res_stride;
+  *rows = c->res_rows;
+  *n_out_slots = (int)c->out_words.size();
+  return B2S_OK;
+}
+
+ColStatsWS*& b2s_int_cols_stats_ws(b2s_cols_s* c) { return c->stats_ws; }
+
 extern "C" int b2s_cols_destroy(b2s_cols_t c) {
   try {  // no C++ exception crosses the C boundary
     if (!c) return B2S_OK;
@@ -453,6 +478,7 @@ extern "C" int b2s_cols_destroy(b2s_cols_t c) {
     for (auto& e : c->ev)
       if (e) cudaEventDestroy(e);
     for (auto& e : c->chunk_ev) cudaEventDestroy(e);
+    b2s_int_colstats_free(c->stats_ws);
     delete c;
     return B2S_OK;
   } catch (const std::exception& e) {

@@ -2,6 +2,8 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <mutex>
+
 #define B2S_HIDDEN __attribute__((visibility("hidden")))
 
 B2S_HIDDEN int b2s_int_fail(int code, const char* fmt, ...);  // sets b2s_last_error(), returns code
@@ -13,6 +15,18 @@ B2S_HIDDEN cudaStream_t b2s_int_copy_stream();                 // the library's 
 B2S_HIDDEN void b2s_int_count_launches(int n);
 struct b2s_plan_s;
 B2S_HIDDEN int b2s_int_plan_shape(b2s_plan_s* plan, int* n_in, int* out_cols);  // B2S_ERR_STATE unless finalized
+
+// the columns plan as the statistics unit sees it (b2s_columns.cu): its mutex (held by b2s_cols_run_host, and by the
+// statistics calls around everything below), the device-resident result of its last b2s_cols_run_host (slot s at
+// *d_out + s * *stride; *generation counts the host runs, so a caller can tell that the result was replaced), and the
+// statistics workspace it owns (freed with the plan by b2s_int_colstats_free).  The last two need the mutex held.
+struct b2s_cols_s;
+struct ColStatsWS;
+B2S_HIDDEN std::mutex& b2s_int_cols_mutex(b2s_cols_s* c);
+B2S_HIDDEN int b2s_int_cols_result(b2s_cols_s* c, const char** d_out, long long* stride, long long* rows, int* n_out_slots,
+                                   unsigned long long* generation);
+B2S_HIDDEN ColStatsWS*& b2s_int_cols_stats_ws(b2s_cols_s* c);
+B2S_HIDDEN void b2s_int_colstats_free(ColStatsWS* ws);
 
 // the online table as the scoring kernel's gather loader sees it (b2s_table.cu fills it in)
 struct B2SGather {

@@ -1,1 +1,2 @@
 from . import steps  # noqa: F401
+from .infer import InferOptions  # noqa: F401

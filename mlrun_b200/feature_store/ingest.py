@@ -8,11 +8,17 @@ datastore/targets.py:1856-1868).  Here the steps are walked symbolically over th
 (`FrameProgram`, same per-row semantics) and lowered to ONE columnar device plan (`mlrun_b200.columns`); the frame's
 columns go to the GPU as they are (contiguous typed arrays) and the result columns come back the same way.
 
-Out of scope (control plane / storage): targets, feature-set metadata / stats inference, sources other than a
-DataFrame.  Steps or dtypes the device cannot hold raise `LoweringError`: there is no per-row Python fallback.
+With `infer_options=InferOptions.Stats (| Histogram | Index)` ingest also profiles the result like the reference's
+`_infer_from_static_df` -> get_df_stats (feature_store/api.py:1162-1196), on the device while the result is still there
+(`infer.py`), into `fset.status.stats` / `get_stats_table()`.  The default here is `InferOptions.Null` (the reference's is
+`InferOptions.default()`).
+
+Out of scope (control plane / storage): targets, schema and preview inference, sources other than a DataFrame or columns.
+Steps or dtypes the device cannot hold raise `LoweringError`: there is no per-row Python fallback.
 """
 
 import math
+import types
 
 import numpy as np
 
@@ -20,6 +26,8 @@ from .. import _native as nat
 from ..columns import F32, I32, I64, ColumnsPlan
 from ..lowering import LoweringError
 from ..serving.resolve import MLRunInvalidArgumentError
+from . import infer
+from .infer import InferOptions
 
 _INT_DTYPES = ("int8", "int16", "int32", "uint8", "uint16", "bool")
 
@@ -316,6 +324,7 @@ class IngestPlan:
         self.violations = {}
         self.unmatched = {}
         self.stats = None
+        self.df_stats = None
 
     @property
     def out_names(self):
@@ -357,9 +366,10 @@ class IngestPlan:
                 out[name] = block[:, j]
         return out
 
-    def run(self, df, reference_dtypes=False):
+    def run(self, df, reference_dtypes=False, infer_options=0):
         """transform the frame; returns a new DataFrame with the same index.  `reference_dtypes=True` widens integer
-        results to int64 (what a frame re-assembled from Python ints has) at the price of a host-side copy."""
+        results to int64 (what a frame re-assembled from Python ints has) at the price of a host-side copy.  With the
+        InferOptions.Stats bit, `self.df_stats` is get_df_stats of the returned frame (else None)."""
         import pandas as pd
 
         if not _same_labels_and_dtypes(df, getattr(self, "_seen", None)):  # a frame like one already checked skips the walk
@@ -369,7 +379,11 @@ class IngestPlan:
         n = len(df)
         ins, _keep = self._inputs(df)
         data, bufs, block, layout = self._run_arrays(ins, n, reference_dtypes)
+        self._describe(data, n, df.index, infer_options)
         return self._assemble(data, bufs, block, layout, n, df.index)
+
+    def _describe(self, data, n, index, infer_options):
+        self.df_stats = infer.describe(self, data, n, index, infer_options) if infer_options & InferOptions.Stats else None
 
     def _run_arrays(self, ins, n, reference_dtypes=False):
         """{input slot: contiguous column array} -> ({result column: array}, landing views, their pinned block, offsets):
@@ -421,12 +435,13 @@ class IngestPlan:
                 int(self.counters[cnt]) for cnt, name, v in self.checks if v in step._validators.values())
         return data, bufs, block, layout
 
-    def run_columns(self, columns, reference_dtypes=False):
+    def run_columns(self, columns, reference_dtypes=False, infer_options=0, index=None):
         """columnar twin of `run` (SURVEY 8(f) #1: "Arrow/DLPack in, Arrow/Parquet-ready columns out"): `columns` maps every
         schema column to a contiguous 1-D array of its dtype (numpy, or anything `columnar.as_columns` understands: Arrow
         tables / record batches, DLPack producers); returns a `columnar.ColumnBatch` whose arrays live in one pinned block.
         No pandas object is built or taken apart; pinned inputs (`columnar.pinned_columns`) cross PCIe at full speed and
-        frames of 128 Ki rows and more are pipelined in row ranges."""
+        frames of 128 Ki rows and more are pipelined in row ranges.  `index` ({entity: array}) is what the statistics of
+        `infer_options` describe as the batch's index columns (none: the row numbers, as for a frame's RangeIndex)."""
         from . import columnar
 
         cols = columnar.as_columns(columns)
@@ -450,6 +465,7 @@ class IngestPlan:
                 raise ValueError("columns of different lengths")
             ins[self.prog.in_slot[name]] = a
         data, _bufs, block, _layout = self._run_arrays(ins, n or 0, reference_dtypes)
+        self._describe(data, n or 0, index or {}, infer_options)
         return columnar.ColumnBatch(data, n or 0, block)
 
     def _assemble(self, data, bufs, block, layout, n, index):
@@ -556,6 +572,16 @@ class FeatureSet:
         self._graph.engine = "sync"  # steps are only resolved here; the device plan replaces the executor
         self._plan = None
         self._plan_key = None
+        self.status = types.SimpleNamespace(stats={})
+
+    def get_stats_table(self):
+        """feature_set.py:853-856: the statistics of the last ingest with InferOptions.Stats as a frame (one row per
+        column), None when there are none"""
+        import pandas as pd
+
+        if self.status.stats:
+            return pd.DataFrame.from_dict(self.status.stats, orient="index")
+        return None
 
     @property
     def graph(self):
@@ -626,8 +652,13 @@ class FeatureSet:
                                  if f.validator is not None and (not o.columns or k in o.columns)}
         return objs
 
-    def ingest(self, source=None, targets=None, namespace=None, return_df=True, reference_dtypes=False, **kwargs):
-        """DataFrame -> transformed DataFrame through one device plan (targets are out of scope: pass none)"""
+    def ingest(self, source=None, targets=None, namespace=None, return_df=True, reference_dtypes=False,
+               infer_options=InferOptions.Null, **kwargs):
+        """DataFrame -> transformed DataFrame through one device plan (targets are out of scope: pass none).
+        `infer_options` (InferOptions bits): Stats fills `status.stats` with get_df_stats of the result, computed on the
+        device; Histogram adds the 20-bin histograms; Index describes the index (entities, else the row numbers) first.
+        Entities / Features / Preview (schema and preview inference) are accepted and ignored.  The default is Null:
+        pass InferOptions.default() for what the reference's ingest does."""
         if targets:
             raise LoweringError("targets are storage (out of scope): ingest returns the frame")
         from . import columnar
@@ -643,8 +674,10 @@ class FeatureSet:
                 self.validate_steps(namespace)
                 self._plan = lower_steps(self._step_objects(namespace), schema)
                 self._plan_key = ("columns", schema)
-            batch = self._plan.run_columns(cols, reference_dtypes=reference_dtypes)
+            batch = self._plan.run_columns(cols, reference_dtypes=reference_dtypes, infer_options=infer_options, index=carried)
             batch.index = carried
+            if infer_options & InferOptions.Stats:
+                self.status.stats = self._plan.df_stats
             return batch if return_df else None
         if not (hasattr(source, "columns") and hasattr(source, "index")):
             raise MLRunInvalidArgumentError("illegal source")  # ingestion.py:77-78; only frames are taken here
@@ -656,7 +689,9 @@ class FeatureSet:
             self.validate_steps(namespace)
             self._plan = lower_steps(self._step_objects(namespace), df)
             self._plan_key = (df.columns, list(df.dtypes))
-        out = self._plan.run(df, reference_dtypes=reference_dtypes)
+        out = self._plan.run(df, reference_dtypes=reference_dtypes, infer_options=infer_options)
+        if infer_options & InferOptions.Stats:
+            self.status.stats = self._plan.df_stats
         return out if return_df else None
 
     @property
