@@ -26,9 +26,6 @@ namespace b2s {
 constexpr int kRTMaxCatCols = 16;
 constexpr int kRTCatsInline = 4;   // categories compared as constant operands
 constexpr int kRTMaxCats = 256;
-#ifndef RT_R2_MINB
-#define RT_R2_MINB 4  // resident CTAs the two-rows-per-thread variant is compiled for
-#endif
 
 template <int NCH, int NS>
 struct RTParams {
@@ -115,29 +112,26 @@ struct RowSwizzled {  // 2-D TMA boxes of 32 floats x TR rows, SWIZZLE_128B: chu
   }
 };
 
-// dot products of the chunks [CH0, CH1) of RPT rows with all NS weight columns (the weights, fills and limits
-// are constant-bank / uniform-register operands: with RPT = 2 each is fetched once for two rows)
-template <int NCH, int NS, int CH0, int CH1, int RPT, typename Row>
-__device__ __forceinline__ void rt_slice(const RTParams<NCH, NS>& p, const Row (&xr)[RPT], double (&acc)[RPT][NS]) {
-  constexpr int BATCH = RPT == 1 ? 4 : 2;  // chunks converted before their DFMAs are issued (ILP)
+// dot products of the chunks [CH0, CH1) of a row with all NS weight columns (the weights, fills and limits
+// are constant-bank / uniform-register operands)
+template <int NCH, int NS, int CH0, int CH1, typename Row>
+__device__ __forceinline__ void rt_slice(const RTParams<NCH, NS>& p, const Row& xr, double (&acc)[NS]) {
+  constexpr int BATCH = 4;  // chunks converted before their DFMAs are issued (ILP)
 #pragma unroll
   for (int b = CH0; b < CH1; b += BATCH) {
-    double xd[RPT][BATCH * 4];
+    double xd[BATCH * 4];
 #pragma unroll
     for (int cb = 0; cb < BATCH; ++cb) {
       const int ch = b + cb;
       if (ch < CH1) {
+        const float4 v = xr.chunk(ch);
+        const float xs[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
-        for (int i = 0; i < RPT; ++i) {
-          const float4 v = xr[i].chunk(ch);
-          const float xs[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            const int c = ch * 4 + u;
-            float x = xs[u];
-            x = !(fabsf(x) <= p.lim[c]) ? p.fill[c] : x;  // Imputer / non-input -> +0 (see RTParams)
-            xd[i][cb * 4 + u] = (double)x;
-          }
+        for (int u = 0; u < 4; ++u) {
+          const int c = ch * 4 + u;
+          float x = xs[u];
+          x = !(fabsf(x) <= p.lim[c]) ? p.fill[c] : x;  // Imputer / non-input -> +0 (see RTParams)
+          xd[cb * 4 + u] = (double)x;
         }
       }
     }
@@ -149,9 +143,7 @@ __device__ __forceinline__ void rt_slice(const RTParams<NCH, NS>& p, const Row (
         for (int u = 0; u < 4; ++u) {
           const int c = ch * 4 + u;
 #pragma unroll
-          for (int k = 0; k < NS; ++k)
-#pragma unroll
-            for (int i = 0; i < RPT; ++i) acc[i][k] = fma(p.w[c][k], xd[i][cb * 4 + u], acc[i][k]);
+          for (int k = 0; k < NS; ++k) acc[k] = fma(p.w[c][k], xd[cb * 4 + u], acc[k]);
         }
       }
     }
@@ -175,9 +167,9 @@ __device__ __noinline__ int rt_cat_search(const RTParams<NCH, NS>& p, int cc, fl
 // one-hot columns Q0, Q0+TPR, ... of one row: "onehot(x) . w" is a gather from the shared-memory weight rows.
 // Fully unrolled with literal column slots (the caller's branch on the slice index is warp-uniform), so every
 // table entry is a constant-bank operand and the address arithmetic stays in the uniform datapath.
-template <int NCH, int NS, int Q0, int TPR, int RPT, typename Row>
-__device__ __forceinline__ void rt_cats(const RTParams<NCH, NS>& p, const Row (&xr)[RPT], const double* __restrict__ s_wcat,
-                                        double (&acc)[RPT][NS]) {
+template <int NCH, int NS, int Q0, int TPR, typename Row>
+__device__ __forceinline__ void rt_cats(const RTParams<NCH, NS>& p, const Row& xr, const double* __restrict__ s_wcat,
+                                        double (&acc)[NS]) {
   constexpr int ITERS = (kRTMaxCatCols - Q0 + TPR - 1) / TPR;
   if (p.cats_fast) {  // integer codes first .. first + cnt - 1 in every column: no search, no per-column branch
     const char* wb = reinterpret_cast<const char*>(s_wcat);
@@ -186,26 +178,23 @@ __device__ __forceinline__ void rt_cats(const RTParams<NCH, NS>& p, const Row (&
       const int cc = Q0 + it * TPR;
       if (cc >= p.n_cat_cols) break;
       const typename RTParams<NCH, NS>::CatFast cf = p.catf[cc];
+      float x = xr.at_b(cf.off_b, cf.sw_b);
+      x = (x != x) ? cf.fill : x;
+      const int v = __float2int_rz(x);  // saturating; NaN -> 0 and fails the equality below
+      const unsigned jj = (unsigned)(v - cf.first);
+      const bool miss = ((float)v != x) | (jj >= (unsigned)cf.cnt);
+      const int a = miss ? p.zero_woff_b : cf.woff_b + (int)jj * (NS * 8);
+      if constexpr (NS % 2 == 0) {  // weight rows are 16-byte aligned: LDS.128
 #pragma unroll
-      for (int i = 0; i < RPT; ++i) {
-        float x = xr[i].at_b(cf.off_b, cf.sw_b);
-        x = (x != x) ? cf.fill : x;
-        const int v = __float2int_rz(x);  // saturating; NaN -> 0 and fails the equality below
-        const unsigned jj = (unsigned)(v - cf.first);
-        const bool miss = ((float)v != x) | (jj >= (unsigned)cf.cnt);
-        const int a = miss ? p.zero_woff_b : cf.woff_b + (int)jj * (NS * 8);
-        if constexpr (NS % 2 == 0) {  // weight rows are 16-byte aligned: LDS.128
-#pragma unroll
-          for (int k = 0; k < NS; k += 2) {
-            const double2 w2 = *reinterpret_cast<const double2*>(wb + a + k * 8);
-            acc[i][k] += w2.x;
-            acc[i][k + 1] += w2.y;
-          }
-        } else {
-          const double* wc = reinterpret_cast<const double*>(wb + a);
-#pragma unroll
-          for (int k = 0; k < NS; ++k) acc[i][k] += wc[k];
+        for (int k = 0; k < NS; k += 2) {
+          const double2 w2 = *reinterpret_cast<const double2*>(wb + a + k * 8);
+          acc[k] += w2.x;
+          acc[k + 1] += w2.y;
         }
+      } else {
+        const double* wc = reinterpret_cast<const double*>(wb + a);
+#pragma unroll
+        for (int k = 0; k < NS; ++k) acc[k] += wc[k];
       }
     }
     return;
@@ -214,31 +203,28 @@ __device__ __forceinline__ void rt_cats(const RTParams<NCH, NS>& p, const Row (&
   for (int it = 0; it < ITERS; ++it) {
     const int cc = Q0 + it * TPR;
     if (cc >= p.n_cat_cols) break;
-#pragma unroll
-    for (int i = 0; i < RPT; ++i) {
-      float x = xr[i].at2(p.cat_off[cc], p.cat_sw[cc]);
-      x = (x != x) ? p.cat_fill[cc] : x;
-      int j;
-      if (p.cat_dense[cc]) {  // integer codes first, first+1, ...: the index is a conversion
-        const int v = __float2int_rz(x);  // saturating; NaN -> 0 and fails the equality below
-        const unsigned jj = (unsigned)(v - p.cat_first[cc]);
-        j = ((float)v == x && jj < (unsigned)p.cat_cnt[cc]) ? p.cat_base[cc] + (int)jj : p.n_cat;  // n_cat: the zero row
-      } else {
-        j = rt_cat_search(p, cc, x);
-      }
-      const double* wc = s_wcat + (size_t)j * NS;
-#pragma unroll
-      for (int k = 0; k < NS; ++k) acc[i][k] += wc[k];
+    float x = xr.at2(p.cat_off[cc], p.cat_sw[cc]);
+    x = (x != x) ? p.cat_fill[cc] : x;
+    int j;
+    if (p.cat_dense[cc]) {  // integer codes first, first+1, ...: the index is a conversion
+      const int v = __float2int_rz(x);  // saturating; NaN -> 0 and fails the equality below
+      const unsigned jj = (unsigned)(v - p.cat_first[cc]);
+      j = ((float)v == x && jj < (unsigned)p.cat_cnt[cc]) ? p.cat_base[cc] + (int)jj : p.n_cat;  // n_cat: the zero row
+    } else {
+      j = rt_cat_search(p, cc, x);
     }
+    const double* wc = s_wcat + (size_t)j * NS;
+#pragma unroll
+    for (int k = 0; k < NS; ++k) acc[k] += wc[k];
   }
 }
 
 // slice q of a row: the dot products over its share of the LIVE leading chunks + its share of the one-hot columns.
 // The slice index is warp-uniform; each case has compile-time column indices (constant operands); the row's one-hot
 // columns are dealt round-robin to its threads.
-template <int NCH, int NS, int TPR, int LIVE, int RPT, typename Row>
-__device__ __forceinline__ void rt_row_slices(const RTParams<NCH, NS>& p, int q, const Row (&xr)[RPT], const double* __restrict__ s_wcat,
-                                              double (&acc)[RPT][NS]) {
+template <int NCH, int NS, int TPR, int LIVE, typename Row>
+__device__ __forceinline__ void rt_row_slices(const RTParams<NCH, NS>& p, int q, const Row& xr, const double* __restrict__ s_wcat,
+                                              double (&acc)[NS]) {
   static_assert(LIVE % TPR == 0, "live chunks must split evenly over the row's threads");
   constexpr int CPT = LIVE / TPR;
   if (TPR == 1 || q == 0) {
@@ -315,12 +301,10 @@ __device__ __noinline__ void rt_generic_epilogue(const RTParams<NCH, NS>& p, con
 }
 
 // LM: how tiles reach shared memory -- 0 LDGSTS (cp.async), 1 one TMA bulk copy per row, 2 TMA tensor-map boxes (swizzled)
-// RPT: rows per thread (2 only with LM = 2): a tile of TR rows is worked on by TR / RPT * TPR threads
-template <int NCH, int NS, int TPR, int LM, int RPT = 1>
-__global__ void __launch_bounds__(128 * TPR / RPT, RPT == 2 ? RT_R2_MINB : (TPR >= 4 ? 2 : (TPR == 2 ? 3 : 4)))
+template <int NCH, int NS, int TPR, int LM>
+__global__ void __launch_bounds__(128 * TPR, TPR == 2 ? 3 : 4)
     rowthread_kernel(const __grid_constant__ RTParams<NCH, NS> p, const __grid_constant__ CUtensorMap tmap) {
   static_assert(NCH % TPR == 0, "chunks must split evenly over the row's threads");
-  static_assert(RPT == 1 || LM == 2, "two rows per thread needs the tensor-map loader (one issuing thread)");
   constexpr int CPT = NCH / TPR;  // chunks per thread
   extern __shared__ __align__(16) unsigned char smem[];
   uint64_t* s_bar = reinterpret_cast<uint64_t*>(smem);  // 4 mbarriers (bulk variant); 64 bytes reserved
@@ -343,9 +327,8 @@ __global__ void __launch_bounds__(128 * TPR / RPT, RPT == 2 ? RT_R2_MINB : (TPR 
   const int S = p.stages;
   const int tile_words = (LM == 2) ? TR * NCH * 4 : TR * p.pitch;
   const int64_t n_tiles = (p.n_rows + TR - 1) / TR;
-  const int TRT = TR / RPT;     // threads per slice; thread r works on rows r, r + TRT, ...
-  const int q = tid / TRT;      // slice of the row (warp-uniform: TRT is a multiple of 32)
-  const int r = tid - q * TRT;  // first row inside the tile
+  const int q = tid / TR;      // slice of the row (warp-uniform: TR is a multiple of 32)
+  const int r = tid - q * TR;  // row inside the tile
 
   // (row, chunk) walk of the tile loader without per-iteration division
   const int cprv = p.vec_ok ? (p.n_in >> 2) : p.n_in;  // units per row: 16-byte chunks or 4-byte words
@@ -498,27 +481,21 @@ __global__ void __launch_bounds__(128 * TPR / RPT, RPT == 2 ? RT_R2_MINB : (TPR 
     const int live_rows = (int)(p.n_rows - row0 < (int64_t)TR ? p.n_rows - row0 : (int64_t)TR);  // uniform: rows of this tile
     const bool any_live = r < live_rows;  // rows past the end were zero-filled (TMA) or are skipped
     using Row = typename std::conditional<LM == 2, RowSwizzled, RowPadded>::type;
-    Row xr[RPT];
-#pragma unroll
-    for (int i = 0; i < RPT; ++i) {
-      const int ri = r + i * TRT;
-      if constexpr (LM == 2) {
-        xr[i].box0 = tile + ri * 32;
-        xr[i].box_words = TR * 32;
-        xr[i].r7s = (r & 7) << 2;  // TRT is a multiple of 8: every row of the thread has the same swizzle phase
-      } else {
-        xr[i].xr = tile + ri * p.pitch;
-      }
+    Row xr;
+    if constexpr (LM == 2) {
+      xr.box0 = tile + r * 32;
+      xr.box_words = TR * 32;
+      xr.r7s = (r & 7) << 2;
+    } else {
+      xr.xr = tile + r * p.pitch;
     }
-    double acc[RPT][NS];
+    double acc[NS];
 #pragma unroll
-    for (int i = 0; i < RPT; ++i)
-#pragma unroll
-      for (int k = 0; k < NS; ++k) acc[i][k] = 0.0;
+    for (int k = 0; k < NS; ++k) acc[k] = 0.0;
     if (any_live) {
       // trailing chunks without a model input are not multiplied at all: the live chunks are split evenly over the row's
       // threads (a uniform branch picks the fully unrolled version for 0, 2 or 4 skipped chunks)
-      if constexpr (LM == 2 && RPT == 1 && NCH >= 8 && (TPR == 1 || TPR == 2)) {  // (the tensor-map variants only: build time)
+      if constexpr (LM == 2 && NCH >= 8 && (TPR == 1 || TPR == 2)) {  // (the tensor-map variants only: build time)
         if (p.dead_tail >= 4) rt_row_slices<NCH, NS, TPR, NCH - 4>(p, q, xr, s_wcat, acc);
         else if (p.dead_tail >= 2) rt_row_slices<NCH, NS, TPR, NCH - 2>(p, q, xr, s_wcat, acc);
         else rt_row_slices<NCH, NS, TPR, NCH>(p, q, xr, s_wcat, acc);
@@ -529,55 +506,47 @@ __global__ void __launch_bounds__(128 * TPR / RPT, RPT == 2 ? RT_R2_MINB : (TPR 
     if (TPR > 1) {  // combine the row's slices in a fixed order (deterministic fp64 sum)
       double* s_part_cur = s_part + (one_sync ? (size_t)(iter & 1) * part_words : 0);
       if (q > 0) {
+        double* part = s_part_cur + ((size_t)(q - 1) * 128 + r) * NS;
 #pragma unroll
-        for (int i = 0; i < RPT; ++i) {
-          double* part = s_part_cur + ((size_t)(q - 1) * 128 + r + i * TRT) * NS;
-#pragma unroll
-          for (int k = 0; k < NS; ++k) part[k] = acc[i][k];
-        }
+        for (int k = 0; k < NS; ++k) part[k] = acc[k];
       }
       __syncthreads();
       if (one_sync) issue_bulk(stage, (t + (int64_t)S * gridDim.x) * TR);  // every read of this stage is behind the barrier
       if (q == 0) {
 #pragma unroll
-        for (int i = 0; i < RPT; ++i)
+        for (int qq = 1; qq < TPR; ++qq) {
+          const double* o = s_part_cur + ((size_t)(qq - 1) * 128 + r) * NS;
 #pragma unroll
-          for (int qq = 1; qq < TPR; ++qq) {
-            const double* o = s_part_cur + ((size_t)(qq - 1) * 128 + r + i * TRT) * NS;
-#pragma unroll
-            for (int k = 0; k < NS; ++k) acc[i][k] += o[k];
-          }
+          for (int k = 0; k < NS; ++k) acc[k] += o[k];
+        }
       }
     }
+    const int64_t row = row0 + r;
+    if (q == 0 && r < live_rows) {
+      uint32_t st = 0;
 #pragma unroll
-    for (int i = 0; i < RPT; ++i) {
-      const int64_t row = row0 + (r + i * TRT);
-      if (q == 0 && r + i * TRT < live_rows) {
-        uint32_t st = 0;
+      for (int k = 0; k < NS; ++k) {
+        acc[k] += p.bias[k];
+        st |= (fabs(acc[k]) <= 1.7976931348623157e308) ? 0u : 1u;
+      }
+      if (LM == 1) st |= ((unknown_bits >> stage) & 1u) << 2;  // B2S_ROW_UNKNOWN_KEY
+      if (p.fast_epilogue) {
+        if (p.vote_kind == 1) {  // VotingEnsemble._mean_vote: sum_m w[m] * pred[m], model order
+          double s = 0.0;
 #pragma unroll
-        for (int k = 0; k < NS; ++k) {
-          acc[i][k] += p.bias[k];
-          st |= (fabs(acc[i][k]) <= 1.7976931348623157e308) ? 0u : 1u;
-        }
-        if (LM == 1) st |= ((unknown_bits >> stage) & 1u) << 2;  // B2S_ROW_UNKNOWN_KEY
-        if (p.fast_epilogue) {
-          if (p.vote_kind == 1) {  // VotingEnsemble._mean_vote: sum_m w[m] * pred[m], model order
-            double s = 0.0;
-#pragma unroll
-            for (int k = 0; k < NS; ++k) s = __dadd_rn(s, __dmul_rn(acc[i][k], p.vote_w[k]));
-            store_word(p, row, 0, __float_as_uint((float)s));
-          } else {
-#pragma unroll
-            for (int k = 0; k < NS; ++k)
-              if (k < p.n_models) store_word(p, row, k, __float_as_uint((float)acc[i][k]));
-          }
-          if (p.status) p.status[row] = (int32_t)st;
+          for (int k = 0; k < NS; ++k) s = __dadd_rn(s, __dmul_rn(acc[k], p.vote_w[k]));
+          store_word(p, row, 0, __float_as_uint((float)s));
         } else {
-          double sl[NS];
 #pragma unroll
-          for (int k = 0; k < NS; ++k) sl[k] = acc[i][k];
-          rt_generic_epilogue(p, sl, row, st);
+          for (int k = 0; k < NS; ++k)
+            if (k < p.n_models) store_word(p, row, k, __float_as_uint((float)acc[k]));
         }
+        if (p.status) p.status[row] = (int32_t)st;
+      } else {
+        double sl[NS];
+#pragma unroll
+        for (int k = 0; k < NS; ++k) sl[k] = acc[k];
+        rt_generic_epilogue(p, sl, row, st);
       }
     }
     ++stage;

@@ -25,10 +25,7 @@
 #include "../../include/b200serve.h"
 #include "b2s_internal.h"
 #include "b2s_device.cuh"
-#include "b2s_rowwarp.cuh"
 #include "b2s_rowthread.cuh"
-#include "b2s_rowmma.cuh"
-#include "b2s_trees2.cuh"
 #include "b2s_trees3.cuh"
 #include "b2s_dense.cuh"
 #include <nvtx3/nvToolsExt.h>  // header-only: ranges cost nothing unless a profiler is attached
@@ -168,36 +165,24 @@ struct b2s_plan_s {
   size_t blob_bytes = 0;
   int grid = 0, block = 0;
   int kernels_per_batch = 1;
-  // row-warp kernel (register-resident linear path)
-  bool rw_ok = false;
-  int rw_L = 0, rw_CPL = 1, rw_NS = 0, rw_U = 0, rw_CS = 0, rw_grid = 0, rw_smem = 0;
-  RWParams rw{};
   // row-thread kernel (constant-bank operands)
   bool rt_ok = false;
   int rt_cat_cols = 0;  // one-hot source columns of the row-thread plan
-  int rt_NCH = 0, rt_NS = 0, rt_TPR = 1, rt_grid = 0, rt_smem = 0, rt_tile_rows = 128, rt_pitch = 0, rt_stages = 2, rt_RPT = 1;
-  // DMMA variant of the row kernel (b2s_rowmma.cuh): tensor-map launches of plans with 32 / 64 columns
-  bool rm_ok = false;
-  int rm_warps = 8, rm_stages = 3, rm_smem = 0;
+  int rt_NCH = 0, rt_NS = 0, rt_grid = 0, rt_smem = 0, rt_pitch = 0;
   std::vector<char> rt_blob;  // an RTParams<NCH, NS>
   // fused ensemble-merge targets (P2P)
   std::vector<void*> peers;
   int64_t peer_off = 0;
   struct b2s_comm_s* comm = nullptr;  // attached merge communicator (double-buffered targets + completion flags)
-  // shared-memory-resident tree kernel
-  bool t2_ok = false;
-  int t2_NS = 1, t2_grid = 0, t2_block = 512, t2_smem = 0;
-  T2Params t2{};
-  char* d_t2_blob = nullptr;
-  // per-model predictions between trees_model_kernel and vote_kernel: one scratch per stream the plan is launched on
+  // trees3 buffers between its three kernels: one scratch per stream the plan is launched on
   // (launches on one stream are ordered; the ring's stream, the library stream and caller streams may overlap)
   struct TreeScratch {
-    double* pred = nullptr;
+    double* pred = nullptr;    // partial sums, column-major (trees3_kernel -> t3_vote_kernel)
     int32_t* row_bad = nullptr;
-    uint32_t* xt = nullptr;  // trees3: the batch transposed into tiles (t3_prep_kernel)
+    uint32_t* xt = nullptr;    // the batch transposed into tiles (t3_prep_kernel -> trees3_kernel)
     int64_t rows = 0;
   };
-  std::map<cudaStream_t, TreeScratch> t2_scratch;
+  std::map<cudaStream_t, TreeScratch> t3_scratch;
   std::mutex scratch_mu;
   // dense linear head on the tensor cores (b2s_dense.cu): > 8 scores over <= 128 plain numeric columns
   bool dense_ok = false;
@@ -210,7 +195,6 @@ struct b2s_plan_s {
   T3Prep t3_prep{};
   int t3_prep_smem = 0;
   char* d_t3_blob = nullptr;
-  std::unique_ptr<T3Top> t3_top;  // top levels of every tree as a launch parameter (null: read from shared memory)
   const int32_t* d_t3_col_score = nullptr;
   // host staging for run_host
   char* h_stage_in = nullptr;
@@ -288,37 +272,6 @@ static cudaError_t launch_plan(b2s_plan_s* p, const KParams& kp, int grid, int b
   return cudaErrorInvalidValue;
 }
 
-constexpr int rw_u(int L, int CPL, int NS) {
-  // row slots in flight per lane: bounded by the butterfly (U*NS <= L) and by the register budget
-  int cap = (NS >= 8 ? 2 : (NS >= 4 ? 4 : 8)) / CPL;
-  int u = L / NS < cap ? L / NS : cap;
-  return u < 1 ? 1 : u;
-}
-
-template <int L, int CPL, int NS, int CS>
-static cudaError_t launch_rw_t(const RWParams& rp, int grid, int smem, cudaStream_t st, bool query, int* occ) {
-  constexpr int U = rw_u(L, CPL, NS);
-  if (query) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, rowwarp_kernel<L, CPL, NS, U, CS>, 128, smem);
-  rowwarp_kernel<L, CPL, NS, U, CS><<<grid, 128, smem, st>>>(rp);
-  return cudaGetLastError();
-}
-
-static cudaError_t launch_rw(int L, int CPL, int NS, int CS, const RWParams& rp, int grid, int smem, cudaStream_t st,
-                             bool query = false, int* occ = nullptr) {
-#define RW_CASE(l, cp, n, c) \
-  if (L == l && CPL == cp && NS == n && CS == c) return launch_rw_t<l, cp, n, c>(rp, grid, smem, st, query, occ);
-#define RW_SHAPES(c)                                                                          \
-  RW_CASE(8, 1, 1, c) RW_CASE(8, 1, 2, c) RW_CASE(8, 1, 4, c) RW_CASE(8, 1, 8, c)             \
-  RW_CASE(8, 2, 1, c) RW_CASE(8, 2, 2, c) RW_CASE(8, 2, 4, c)                                 \
-  RW_CASE(16, 1, 8, c)                                                                        \
-  RW_CASE(16, 2, 1, c) RW_CASE(16, 2, 2, c) RW_CASE(16, 2, 4, c)                              \
-  RW_CASE(32, 1, 8, c)
-  RW_SHAPES(0) RW_SHAPES(1) RW_SHAPES(2)
-#undef RW_SHAPES
-#undef RW_CASE
-  return cudaErrorInvalidValue;
-}
-
 // cuTensorMapEncodeTiled, resolved at run time (no link-time dependency on libcuda)
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -332,19 +285,6 @@ static EncodeTiledFn tensor_map_encoder() {
       sym = nullptr;
     }
     return reinterpret_cast<EncodeTiledFn>(sym);
-  }();
-  return fn;
-}
-typedef CUresult (*BatchMemOpFn)(CUstream, unsigned int, CUstreamBatchMemOpParams*, unsigned int);
-static BatchMemOpFn stream_batch_memop() {
-  static BatchMemOpFn fn = [] {
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuStreamBatchMemOp", &sym, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-      cudaGetLastError();
-      sym = nullptr;
-    }
-    return reinterpret_cast<BatchMemOpFn>(sym);
   }();
   return fn;
 }
@@ -378,6 +318,8 @@ struct RTTables {  // what rt_build needs from finalize
 
 // threads per row: measured on B200 (profiles/r1_kernel_log.md): 2 beats 1 (more warps) and 4 (combine overhead)
 constexpr int rt_tpr(int NCH) { return NCH >= 8 ? 2 : 1; }
+constexpr int kRTTileRows = 128;  // rows per tile (the launch halves it for small batches)
+constexpr int kRTStages = 2;      // depth of the tile ring
 
 template <int NCH, int NS>
 static void rt_build(b2s_plan_s* p, const RTTables& t) {
@@ -442,51 +384,40 @@ static void rt_build(b2s_plan_s* p, const RTTables& t) {
     int last_live = -1;  // last chunk that holds a model-input column
     for (int c = 0; c < t.n_in; ++c)
       if (((*t.flags)[c] & COL_COPIED) != 0) last_live = c >> 2;
-    r.dead_tail = std::max(0, NCH - 1 - last_live);
-    if (last_live < 0 || getenv("B2S_RT_NOSKIP")) r.dead_tail = 0;  // (A/B runs)
+    r.dead_tail = last_live < 0 ? 0 : std::max(0, NCH - 1 - last_live);
   }
-  if (getenv("B2S_RT_SLOWCATS")) r.cats_fast = 0;
   for (int i = 0; i < r.n_cat; ++i) r.cat_val[i] = (*t.cat_val)[i];
 }
 
-static int rt_load_mode() {  // B2S_TMA: 0 cp.async (LDGSTS), 1 one TMA bulk copy per row, 2 TMA tensor-map boxes (default)
-  static const int mode = getenv("B2S_TMA") ? atoi(getenv("B2S_TMA")) : 2;
-  return mode;
-}
+// the tensor-map loader needs rows of >= 128 bytes that fill the plan's chunks exactly
+static bool rt_tmap_ok(const b2s_plan_s* p) { return p->rt_NCH >= 8 && p->n_in == p->rt_NCH * 4 && tensor_map_encoder() != nullptr; }
 
 struct LaunchCtx {             // per-launch context (launches of one plan may be issued from several threads at once)
   const KParams* k = nullptr;  // merge targets / completion signal of this launch
   bool host_rows = false;      // the rows live in mapped host memory (zero-copy small batches): plain cp.async loads
 };
 
-template <int NCH, int NS, int TPR>
-static cudaError_t rt_launch_tt(b2s_plan_s* p, const void* rows, int64_t stride, int64_t n_rows, void* out, int32_t* status,
-                                int vec_ok, cudaStream_t st, bool query, int* occ, const B2SGather* gather, const LaunchCtx* lc) {
+template <int NCH, int NS>
+static cudaError_t rt_launch_t(b2s_plan_s* p, const void* rows, int64_t stride, int64_t n_rows, void* out, int32_t* status,
+                               int vec_ok, cudaStream_t st, bool query, int* occ, const B2SGather* gather, const LaunchCtx* lc) {
   using P = RTParams<NCH, NS>;
+  constexpr int TPR = rt_tpr(NCH);
   constexpr int LMT = NCH >= 8 ? 2 : 1;  // the tensor-map variants exist for rows of >= 128 bytes
-  constexpr int R2 = NCH >= 8 ? 2 : 1;
   static std::atomic<bool> attr_set{false};  // the dispatcher thread and callers may both get here first
   if (!attr_set) {
     const int cap = (int)G.prop.sharedMemPerBlockOptin;
     cudaError_t e = cudaFuncSetAttribute(rowthread_kernel<NCH, NS, TPR, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(rowthread_kernel<NCH, NS, TPR, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
-    if (e == cudaSuccess && NCH >= 8) {
+    if (e == cudaSuccess && NCH >= 8)
       e = cudaFuncSetAttribute(rowthread_kernel<NCH, NS, TPR, LMT>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
-      if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(rowthread_kernel<NCH, NS, TPR, LMT, R2>, cudaFuncAttributeMaxDynamicSharedMemorySize, cap);
-    }
     if (e != cudaSuccess) return e;
     attr_set = true;
   }
-  const bool tmap_ok = NCH >= 8 && p->n_in == NCH * 4 && tensor_map_encoder() != nullptr;
+  const bool tmap_ok = rt_tmap_ok(p);
   if (query) {  // occupancy of the variant an aligned launch takes
-    const int mode = rt_load_mode() == 2 && !tmap_ok ? 1 : rt_load_mode();
-    if (mode == 2 && p->rt_RPT == 2)
-      return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, rowthread_kernel<NCH, NS, TPR, LMT, R2>,
-                                                           p->rt_tile_rows / 2 * TPR, p->rt_smem);
-    if (mode == 2)
-      return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, rowthread_kernel<NCH, NS, TPR, LMT>, p->rt_tile_rows * TPR, p->rt_smem);
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, rowthread_kernel<NCH, NS, TPR, 0>, p->rt_tile_rows * TPR, p->rt_smem);
+    if (tmap_ok)
+      return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, rowthread_kernel<NCH, NS, TPR, LMT>, kRTTileRows * TPR, p->rt_smem);
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, rowthread_kernel<NCH, NS, TPR, 0>, kRTTileRows * TPR, p->rt_smem);
   }
   P r = *reinterpret_cast<const P*>(p->rt_blob.data());
   r.rows = (const char*)rows;
@@ -501,8 +432,9 @@ static cudaError_t rt_launch_tt(b2s_plan_s* p, const void* rows, int64_t stride,
   for (int g = 0; g < r.n_peers; ++g) r.peers[g] = lk ? lk->peers[g] : (float*)p->peers[g];
   r.sig = lk ? lk->sig : MergeSig{};
   r.pitch = p->rt_pitch;
-  r.stages = p->rt_stages;
-  int mode = vec_ok ? rt_load_mode() : 0;
+  r.stages = kRTStages;
+  // tile loader: 2 TMA tensor-map boxes, 1 one TMA bulk copy per row, 0 cp.async (LDGSTS) for unaligned or host-resident rows
+  int mode = vec_ok ? 2 : 0;
   if (lc && lc->host_rows) mode = 0;
   if (mode == 2 && !tmap_ok) mode = 1;
   if (gather) {  // rows come from the online table: one bulk copy per row, source found by key inside the kernel
@@ -523,31 +455,18 @@ static cudaError_t rt_launch_tt(b2s_plan_s* p, const void* rows, int64_t stride,
         }
       }
   }
-  int rpt = (mode == 2) ? p->rt_RPT : 1;
-  int tr = p->rt_tile_rows;
-  while (tr > 32 * rpt && (n_rows + tr - 1) / tr < (int64_t)G.prop.multiProcessorCount) tr /= 2;
-  const bool mma = mode == 2 && p->rm_ok;  // DMMA variant: warp-private rings of 32-row tiles
-  if (mma) {
-    tr = 32;
-    rpt = 1;
-  }
+  int tr = kRTTileRows;
+  while (tr > 32 && (n_rows + tr - 1) / tr < (int64_t)G.prop.multiProcessorCount) tr /= 2;
   alignas(64) CUtensorMap tmap;
   memset(&tmap, 0, sizeof(tmap));
-  if (mode == 2 && !encode_rows_map(&tmap, rows, n_rows, stride, p->n_in, tr)) {
-    mode = 1;
-    rpt = 1;
-  }
+  if (mode == 2 && !encode_rows_map(&tmap, rows, n_rows, stride, p->n_in, tr)) mode = 1;
   r.tile_rows = tr;
   const int64_t tiles = (n_rows + tr - 1) / tr;
-  static const int grid_mul = getenv("B2S_RT_GRIDMUL") ? std::max(1, atoi(getenv("B2S_RT_GRIDMUL"))) : 1;  // CTA waves (1 = persistent)
-  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)p->rt_grid * grid_mul, tiles));
+  const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(p->rt_grid, tiles));
   r.use_bulk = mode;
-  {
-    // single-barrier tile loop: measured better with 4 score columns (0.0506 vs 0.0512 ms, r2o) and worse with one
-    // (0.0481 vs 0.0454 ms, r2q / r2o): the default follows the number of score columns
-    static const int one_sync = getenv("B2S_RT_ONESYNC") ? atoi(getenv("B2S_RT_ONESYNC")) : -1;
-    r.one_sync = one_sync >= 0 ? one_sync : (NS >= 4 ? 1 : 0);
-  }
+  // single-barrier tile loop: measured better with 4 score columns (0.0506 vs 0.0512 ms, r2o) and worse with one
+  // (0.0481 vs 0.0454 ms, r2q / r2o): it follows the number of score columns
+  r.one_sync = NS >= 4 ? 1 : 0;
   for (int cc = 0; cc < r.n_cat_cols; ++cc) {  // tile-relative position of each categorical column
     const int col = r.cat_col[cc], ch = col >> 2;
     r.cat_off[cc] = mode == 2 ? (ch >> 3) * (tr * 32) + (col & 3) : col;
@@ -555,33 +474,13 @@ static cudaError_t rt_launch_tt(b2s_plan_s* p, const void* rows, int64_t stride,
     r.catf[cc].off_b = r.cat_off[cc] * 4;
     r.catf[cc].sw_b = r.cat_sw[cc] * 4;
   }
-  if (mode == 2 && mma) {
-    r.stages = p->rm_stages;
-    const int64_t per_cta = (tiles + G.prop.multiProcessorCount - 1) / G.prop.multiProcessorCount;  // tiles a CTA will see
-    const int warps = (int)std::max<int64_t>(1, std::min<int64_t>(p->rm_warps, per_cta));
-    const int mgrid = (int)std::max<int64_t>(1, std::min<int64_t>(G.prop.multiProcessorCount, tiles));
-    return rowmma_launch(NCH, NS, &r, &tmap, mgrid, warps, (size_t)p->rm_smem, st);
-  }
-  if (mode == 2 && rpt == 2)
-    rowthread_kernel<NCH, NS, TPR, LMT, R2><<<grid, tr / 2 * TPR, p->rt_smem, st>>>(r, tmap);
-  else if (mode == 2)
+  if (mode == 2)
     rowthread_kernel<NCH, NS, TPR, LMT><<<grid, tr * TPR, p->rt_smem, st>>>(r, tmap);
   else if (mode == 1)
     rowthread_kernel<NCH, NS, TPR, 1><<<grid, tr * TPR, p->rt_smem, st>>>(r, tmap);
   else
     rowthread_kernel<NCH, NS, TPR, 0><<<grid, tr * TPR, p->rt_smem, st>>>(r, tmap);
   return cudaGetLastError();
-}
-
-template <int NCH, int NS>
-static cudaError_t rt_launch_t(b2s_plan_s* p, const void* rows, int64_t stride, int64_t n_rows, void* out, int32_t* status,
-                               int vec_ok, cudaStream_t st, bool query, int* occ, const B2SGather* gather, const LaunchCtx* lc) {
-  if (p->rt_TPR == 1) return rt_launch_tt<NCH, NS, 1>(p, rows, stride, n_rows, out, status, vec_ok, st, query, occ, gather, lc);
-  if (NCH >= 8 && p->rt_TPR == 2)
-    return rt_launch_tt<NCH, NS, (NCH >= 8 ? 2 : 1)>(p, rows, stride, n_rows, out, status, vec_ok, st, query, occ, gather, lc);
-  if (NCH >= 16 && p->rt_TPR == 4)
-    return rt_launch_tt<NCH, NS, (NCH >= 16 ? 4 : 1)>(p, rows, stride, n_rows, out, status, vec_ok, st, query, occ, gather, lc);
-  return cudaErrorInvalidValue;
 }
 
 #define RT_DISPATCH(FN, ...)                                                              \
@@ -879,8 +778,8 @@ static int32_t host_key(float x) {
   return b ^ ((b >> 31) & 0x7fffffff);
 }
 
-// Lower a MODE_TREES plan to parts (b2s_trees3.cuh).  Leaves p->t3_ok false when the plan does not qualify (the caller
-// then falls back to the round-1 kernels); returns an error only for CUDA failures.
+// Lower a MODE_TREES plan to parts (b2s_trees3.cuh).  Leaves p->t3_ok false when the plan does not qualify (it then runs
+// on the generic rows_kernel<TREES>); returns an error only for CUDA failures.
 static int t3_build(b2s_plan_s* p, const KParams& k, bool any_fill) {
   const int n_in = p->n_in, M = (int)p->models.size();
   const int sms = G.prop.multiProcessorCount;
@@ -946,10 +845,8 @@ static int t3_build(b2s_plan_s* p, const KParams& k, bool any_fill) {
       }
   int W = 0;
   {
-    const char* wenv = getenv("B2S_T3_WARPS");
-    const int w_lo = wenv ? std::max(4, std::min(kMaxW, atoi(wenv))) : 16, w_hi = wenv ? w_lo : kMaxW;
     double best = 1e300;
-    for (int w = w_lo; w <= w_hi; ++w) {
+    for (int w = 16; w <= kMaxW; ++w) {
       const int cap = capacity(w);
       if (cap < 1) continue;
       double cost = n_lin_cols > 0 ? 2.0 : 0.0;
@@ -1111,7 +1008,7 @@ static int t3_build(b2s_plan_s* p, const KParams& k, bool any_fill) {
   tb.data.resize(o_parts + sizeof(T3Part) * P);
   CUDA_TRY(cudaMalloc(&p->d_t3_blob, tb.data.size()));
   std::vector<T3Part> dev(P);
-  int cta0 = 0, top0 = 0;
+  int cta0 = 0;
   for (int i = 0; i < P; ++i) {
     T3Part& d = dev[i];
     d.nodes = parts[i].n_trees ? (const uint2*)(p->d_t3_blob + o_nodes[i]) : nullptr;
@@ -1121,23 +1018,7 @@ static int t3_build(b2s_plan_s* p, const KParams& k, bool any_fill) {
     d.col0 = parts[i].col0;
     d.cta0 = cta0;
     d.n_ctas = n_ctas[i];
-    d.top0 = top0;
-    top0 += parts[i].n_trees;
     cta0 += n_ctas[i];
-  }
-  // the top three levels as a launch parameter (constant bank) when every tree fits and has them
-  p->t3_top.reset();
-  {
-    const char* tenv = getenv("B2S_T3_TOPC");
-    // measured (r2h): 0.3187 vs 0.3209 ms per 256 Ki events on configs[2] -- within noise, so it stays opt-in
-    if (D >= 3 && top0 <= kT3TopTrees && tenv && atoi(tenv) == 1 && !getenv("B2S_T3_UNROLL")) {
-      p->t3_top.reset(new T3Top);
-      memset(p->t3_top.get(), 0, sizeof(T3Top));
-      int q0 = 0;
-      for (auto& hp : parts)
-        for (int q = 0; q < hp.n_trees; ++q, ++q0)
-          for (int j = 0; j < 7; ++j) p->t3_top->n[(size_t)q0 * 7 + j] = hp.nodes[(size_t)q * NN + 1 + j];
-    }
   }
   memcpy(tb.data.data() + o_parts, dev.data(), sizeof(T3Part) * P);
   CUDA_TRY(cudaMemcpy(p->d_t3_blob, tb.data.data(), tb.data.size(), cudaMemcpyHostToDevice));
@@ -1149,7 +1030,6 @@ static int t3_build(b2s_plan_s* p, const KParams& k, bool any_fill) {
   t.n_in = n_in;
   t.n_parts = P;
   t.warps = W;
-  t.unroll = getenv("B2S_T3_UNROLL") ? atoi(getenv("B2S_T3_UNROLL")) : kT3U;
   t.xt_words = xt_words;
   size_t off = 0;
   auto take = [&](size_t bytes, size_t al) {
@@ -1385,66 +1265,6 @@ extern "C" int b2s_plan_finalize(b2s_plan_t p) {
       for (int u = 0; fast && u < 4; ++u) fast = (flags[ch * 4 + u] == COL_COPIED);
       chunk_kind[ch] = fast ? 0 : 1;
     }
-    // ---- row-warp kernel tables (linear plans over <= 128 columns without MapValues)
-    std::vector<float> rw_fill;
-    std::vector<uint32_t> rw_copied;
-    std::vector<double> rw_w;
-    std::vector<int32_t> rw_csrc, rw_ccomp, rw_cbase, rw_cn;
-    uint32_t rw_cat_pos_mask = 0;
-    {
-      const int nch = (n_in + 3) / 4;
-      int L, CPL;
-      if (NS <= 4) {
-        L = nch <= 16 ? 8 : 16;
-        CPL = nch <= 8 ? 1 : 2;
-      } else {
-        L = nch <= 8 ? 8 : (nch <= 16 ? 16 : 32);
-        CPL = 1;
-      }
-      std::vector<int> cat_cols;
-      int max_cats = 0;
-      if (p->mode == MODE_LINEAR)
-        for (int c = 0; c < n_in; ++c)
-          if (cat_off[c + 1] > cat_off[c]) {
-            cat_cols.push_back(c);
-            max_cats = std::max(max_cats, cat_off[c + 1] - cat_off[c]);
-          }
-      const int CS = (int)((cat_cols.size() + L - 1) / L);
-      const bool env_off = getenv("B2S_NO_ROWWARP") != nullptr;
-      if (!env_off && p->mode == MODE_LINEAR && !any_map && (n_in % 4) == 0 && nch <= L * CPL && NS <= 8 && CS <= 2 && max_cats <= 64) {
-        p->rw_ok = true;
-        p->rw_L = L;
-        p->rw_CPL = CPL;
-        p->rw_NS = NS;
-        p->rw_CS = CS;
-        p->rw_U = rw_u(L, CPL, NS);
-        const int npos = L * CPL;
-        rw_fill.assign((size_t)npos * 4, std::numeric_limits<float>::quiet_NaN());
-        rw_copied.assign(npos, 0);
-        rw_w.assign((size_t)npos * 4 * NS, 0.0);
-        auto pos_of = [&](int c) { const int ch = c / 4; return (ch / L) * L + (ch % L); };
-        for (int c = 0; c < n_in; ++c) {
-          const int pos = pos_of(c), u = c % 4;
-          rw_fill[(size_t)pos * 4 + u] = p->fill[c];
-          if (flags[c] & COL_COPIED) rw_copied[pos] |= (1u << u);
-          for (int kk = 0; kk < NS; ++kk) rw_w[((size_t)pos * 4 + u) * NS + kk] = wnum[(size_t)c * NS + kk];
-        }
-        const int slots = std::max(CS, 1);
-        rw_csrc.assign((size_t)slots * L, -1);
-        rw_ccomp.assign((size_t)slots * L, 0);
-        rw_cbase.assign((size_t)slots * L, 0);
-        rw_cn.assign((size_t)slots * L, 0);
-        for (size_t i = 0; i < cat_cols.size(); ++i) {
-          const int c = cat_cols[i];
-          const size_t at = (i / L) * L + (i % L);
-          rw_csrc[at] = pos_of(c);
-          rw_cat_pos_mask |= 1u << ((pos_of(c) / L) * 4 + (c % 4));
-          rw_ccomp[at] = c % 4;
-          rw_cbase[at] = cat_off[c];
-          rw_cn[at] = cat_off[c + 1] - cat_off[c];
-        }
-      }
-    }
     // ---- dense head (tcgen05): linear scorers with more than 8 scores in total over plain numeric columns.  The float64
     // coefficients become three tf32 terms wh + wm + wl (11 significant bits each, 33 in total); W^T rows padded to 16 / 32
     std::vector<float> dense_wh, dense_wm, dense_wl;
@@ -1491,9 +1311,7 @@ extern "C" int b2s_plan_finalize(b2s_plan_t p) {
                  o_bias = bb.add(bias), o_models = bb.add(descs), o_classes = bb.add(classes),
                  o_votew = bb.add(p->vote_w), o_wgen = bb.add(wgen), o_nodes = bb.add(nodes), o_leaf = bb.add(leaf),
                  o_troot = bb.add(tree_root), o_tslot = bb.add(tree_slot), o_tscale = bb.add(tree_scale),
-                 o_chunk = bb.add(chunk_kind), o_rwfill = bb.add(rw_fill), o_rwcop = bb.add(rw_copied),
-                 o_rww = bb.add(rw_w), o_rwcs = bb.add(rw_csrc), o_rwcc = bb.add(rw_ccomp), o_rwcb = bb.add(rw_cbase),
-                 o_rwcn = bb.add(rw_cn);
+                 o_chunk = bb.add(chunk_kind);
     CUDA_TRY(cudaSetDevice(G.device));
     CUDA_TRY(cudaMalloc(&p->d_blob, bb.data.size()));
     CUDA_TRY(cudaMemcpy(p->d_blob, bb.data.data(), bb.data.size(), cudaMemcpyHostToDevice));
@@ -1664,52 +1482,11 @@ extern "C" int b2s_plan_finalize(b2s_plan_t p) {
     int occ = std::max(1, std::min(blocks_per_sm, smem_cap / std::max(total, 1)));
     p->grid = sms * occ;
 
-    if (p->rw_ok) {
-      RWParams& r = p->rw;
-      memset(&r, 0, sizeof(r));
-      r.n_in = n_in;
-      r.nch = (n_in + 3) / 4;
-      r.out_cols = p->out_cols;
-      r.n_models = M;
-      r.vote_kind = p->vote_kind;
-      r.out_is_int = p->out_is_int;
-      r.n_cat_slots = p->rw_CS;
-      r.n_cat = (int)cat_val.size();
-      bool simple = true;
-      for (auto& m : p->models) simple = simple && m.link == B2S_LINK_IDENTITY && m.n_scores == 1;
-      r.fast_epilogue = (simple && p->vote_kind != B2S_VOTE_MAJORITY) ? 1 : 0;
-      r.fill = (const float*)(B + o_rwfill);
-      r.copied = (const uint32_t*)(B + o_rwcop);
-      r.w = (const double*)(B + o_rww);
-      r.cat_src = (const int32_t*)(B + o_rwcs);
-      r.cat_comp = (const int32_t*)(B + o_rwcc);
-      r.cat_base = (const int32_t*)(B + o_rwcb);
-      r.cat_n = (const int32_t*)(B + o_rwcn);
-      r.cat_val = k.cat_val;
-      r.wcat = k.wcat;
-      r.bias = k.bias;
-      r.vote_w = k.vote_w;
-      r.models = k.models;
-      r.classes = k.classes;
-      p->rw_smem = (int)(align_up((size_t)r.n_cat * 4, 16) + (size_t)(r.n_cat + 1) * NS * 8 + 16);
-      r.cat_pos_mask = rw_cat_pos_mask;
-      int occ = 0;
-      cudaError_t e = launch_rw(p->rw_L, p->rw_CPL, p->rw_NS, p->rw_CS, r, 0, p->rw_smem, nullptr, true, &occ);
-      if (e != cudaSuccess || occ < 1) {
-        cudaGetLastError();
-        p->rw_ok = false;
-      } else {
-        p->rw_grid = sms * occ;
-      }
-    }
     {
-      const char* pick = getenv("B2S_LINEAR_KERNEL");  // rowthread (default) | rowwarp | generic  (A/B runs)
-      const std::string want = pick ? pick : "rowthread";
       int n_cat_cols = 0;
       for (int c = 0; c < n_in; ++c) n_cat_cols += (cat_off[c + 1] > cat_off[c]) ? 1 : 0;
-      if (want != "rowwarp") p->rw_ok = p->rw_ok && (want == "rowwarp");
-      if (want == "rowthread" && p->mode == MODE_LINEAR && !any_map && n_in <= 128 && NS <= 8 &&
-          n_cat_cols <= kRTMaxCatCols && (int)cat_val.size() <= kRTMaxCats) {
+      if (p->mode == MODE_LINEAR && !any_map && n_in <= 128 && NS <= 8 && n_cat_cols <= kRTMaxCatCols &&
+          (int)cat_val.size() <= kRTMaxCats) {
         const int nch = (n_in + 3) / 4;
         p->rt_NCH = nch <= 4 ? 4 : (nch <= 8 ? 8 : (nch <= 16 ? 16 : 32));
         p->rt_NS = NS;
@@ -1722,161 +1499,29 @@ extern "C" int b2s_plan_finalize(b2s_plan_t p) {
         int rpitch = p->rt_NCH * 4 + 4;
         if (((rpitch / 4) & 1) == 0) rpitch += 4;
         p->rt_pitch = rpitch;
-        const char* stg = getenv("B2S_RT_STAGES");
-        p->rt_stages = stg ? std::max(2, std::min(4, atoi(stg))) : 2;
-        const char* tile_env = getenv("B2S_RT_TILE");  // rows per tile: 64 | 128
-        p->rt_tile_rows = tile_env && atoi(tile_env) == 64 ? 64 : 128;
-        const char* rpt_env = getenv("B2S_RT_RPT");  // rows per thread: 1 | 2 (2: tensor-map loads only)
-        p->rt_RPT = rpt_env && atoi(rpt_env) == 2 && p->rt_NCH >= 8 ? 2 : 1;
-        const char* tprs = getenv("B2S_RT_TPR");
-        p->rt_TPR = tprs ? atoi(tprs) : rt_tpr(p->rt_NCH);
-        if (p->rt_TPR != 1 && p->rt_TPR != 2 && p->rt_TPR != 4) p->rt_TPR = 1;
-        while (p->rt_TPR > 1 && (p->rt_NCH < 4 * p->rt_TPR)) p->rt_TPR /= 2;
         {
           const size_t fixed = 1024 + 64 + align_up((size_t)(cat_val.size() + 1) * NS * 8, 16);
-          const size_t part = (size_t)(p->rt_TPR - 1) * 128 * NS * 8;
+          const size_t part = (size_t)(rt_tpr(p->rt_NCH) - 1) * 128 * NS * 8;
           // padded tiles + one partial-sum buffer (LDGSTS / per-row bulk), or swizzled tiles + two (tensor map)
-          const size_t padded = fixed + part + (size_t)p->rt_stages * p->rt_tile_rows * rpitch * 4;
-          const size_t swizzled = fixed + 2 * part + (size_t)p->rt_stages * p->rt_tile_rows * p->rt_NCH * 16;
+          const size_t padded = fixed + part + (size_t)kRTStages * kRTTileRows * rpitch * 4;
+          const size_t swizzled = fixed + 2 * part + (size_t)kRTStages * kRTTileRows * p->rt_NCH * 16;
           p->rt_smem = (int)std::max(padded, swizzled);
         }
         int occ = 0;
         if (p->rt_smem <= smem_cap && rt_launch(p, nullptr, 0, 0, nullptr, nullptr, 0, nullptr, true, &occ) == cudaSuccess && occ >= 1) {
           p->rt_ok = true;
           p->rt_grid = sms * occ;
-          // DMMA variant, opt-in with B2S_RT_MMA=1 (measured slower than the DFMA kernel: profiles/r2_kernel_log.md): 32 or 64
-          // float32 columns, tensor-map loads
-          const char* mma_env = getenv("B2S_RT_MMA");
-          if (mma_env && atoi(mma_env) != 0 && (p->rt_NCH == 8 || p->rt_NCH == 16) && n_in == p->rt_NCH * 4 && tensor_map_encoder()) {
-            const char* we = getenv("B2S_RM_WARPS");
-            const char* se = getenv("B2S_RM_STAGES");
-            p->rm_warps = we ? std::max(1, std::min(kRMMaxWarps, atoi(we))) : 12;
-            p->rm_stages = se ? std::max(2, std::min(kRMMaxStages, atoi(se))) : 2;
-            while (p->rm_warps > 1 && rowmma_smem_bytes(p->rt_NCH, NS, (int)cat_val.size(), p->rm_warps, p->rm_stages) > (size_t)smem_cap) --p->rm_warps;
-            p->rm_smem = (int)rowmma_smem_bytes(p->rt_NCH, NS, (int)cat_val.size(), p->rm_warps, p->rm_stages);
-            if (p->rm_smem <= smem_cap && rowmma_prepare(p->rt_NCH, NS, smem_cap) == cudaSuccess) p->rm_ok = true;
-            else cudaGetLastError();
-          }
         } else {
           cudaGetLastError();
         }
       }
     }
     // ---- round-2 tree path: parts resident in shared memory (b2s_trees3.cuh).  Covers tree ensembles (any number of
-    // score slots per model), ensembles mixing tree and linear scorers, an Imputer in front, and NaN routing.
-    const char* trees_pick = getenv("B2S_TREES");  // 3 (default) | 2 (round-1 kernel) | 0 (generic rows_kernel)  -- A/B runs
-    const int trees_want = trees_pick ? atoi(trees_pick) : 3;
-    if (p->mode == MODE_TREES && identity_schema && !any_map && trees_want == 3) {
+    // score slots per model), ensembles mixing tree and linear scorers, an Imputer in front, and NaN routing.  The plans it
+    // declines (deeper than kT3MaxDepth, more parts than SMs, rows too wide for a part, a schema or MapValues in front) run
+    // on rows_kernel<TREES>.
+    if (p->mode == MODE_TREES && identity_schema && !any_map) {
       if (int rc = t3_build(p, k, any_fill)) return rc;
-    }
-    if (!p->t3_ok && trees_want >= 2)
-    if (p->mode == MODE_TREES && !need_expand && getenv("B2S_NO_TREES2") == nullptr) {
-      // re-pack every model as complete heap-ordered trees; one model must fit one CTA's shared memory
-      bool ok = true;
-      std::vector<int> depth(M, 0);
-      size_t max_table = 0;
-      for (int mi = 0; mi < M && ok; ++mi) {
-        auto& m = p->models[mi];
-        if (m.kind != MK_TREES) { ok = false; break; }
-        const int nt = (int)m.tree_slot.size();
-        for (int t = 0; t < nt; ++t) {
-          const int base = m.tree_offset[t];
-          std::vector<std::pair<int, int>> stack{{0, 0}};
-          while (!stack.empty()) {
-            auto [node, d] = stack.back();
-            stack.pop_back();
-            depth[mi] = std::max(depth[mi], d);
-            if (m.feature[base + node] >= 0) {
-              stack.push_back({m.left[base + node], d + 1});
-              stack.push_back({m.right[base + node], d + 1});
-            }
-          }
-        }
-        if (depth[mi] > 8) ok = false;
-        const size_t ni = ((size_t)1 << depth[mi]) - 1, nl = (size_t)1 << depth[mi];
-        max_table = std::max(max_table, align_up((size_t)nt * ni * 8, 16) + (size_t)nt * nl * 8 + (size_t)nt * 4);
-      }
-      const int TR2 = kT2TileRows, G2 = kT2Groups, ST2 = 1;  // one row-major landing tile + one transposed tile
-      const int NS2 = p->NS <= 1 ? 1 : (p->NS <= 4 ? 4 : 0);
-      const size_t part_bytes = (size_t)(G2 - 1) * TR2 * std::max(NS2, 1) * 8;
-      const size_t tiles_bytes = (size_t)ST2 * TR2 * pitch * 4 + (size_t)((n_in + 3) / 4 * 4) * TR2 * 4 + (size_t)TR2 * 4 + 16 + 1024;  // + mbarrier + alignment slack
-      const size_t total2 = align_up(max_table, 16) + align_up(part_bytes, 16) + tiles_bytes;
-      if (ok && NS2 > 0 && total2 <= (size_t)smem_cap && M <= sms) {
-        BlobBuilder tb;
-        std::vector<T2Model> t2m(M);
-        std::vector<size_t> o_nodes(M), o_leaves(M), o_slot(M), o_scale(M);
-        for (int mi = 0; mi < M; ++mi) {
-          auto& m = p->models[mi];
-          const int nt = (int)m.tree_slot.size();
-          const int D = depth[mi];
-          const int ni = (1 << D) - 1, nl = 1 << D;
-          std::vector<HeapNode> hn((size_t)nt * std::max(ni, 1), HeapNode{0, std::numeric_limits<float>::infinity()});
-          std::vector<double> hl((size_t)nt * nl, 0.0);
-          for (int t = 0; t < nt; ++t) {
-            const int base = m.tree_offset[t];
-            struct It { int heap, d, src; };
-            std::vector<It> stack{{0, 0, 0}};
-            while (!stack.empty()) {
-              It it = stack.back();
-              stack.pop_back();
-              const bool leaf = m.feature[base + it.src] < 0;
-              if (it.d == D) {
-                hl[(size_t)t * nl + (it.heap - ni)] = m.leaf_value[base + it.src];
-                continue;
-              }
-              if (leaf) {  // pad: a threshold of +inf sends every finite value left; both sides carry the leaf
-                hn[(size_t)t * ni + it.heap] = HeapNode{0, std::numeric_limits<float>::infinity()};
-                stack.push_back({2 * it.heap + 1, it.d + 1, it.src});
-                stack.push_back({2 * it.heap + 2, it.d + 1, it.src});
-              } else {
-                hn[(size_t)t * ni + it.heap] = HeapNode{m.feature[base + it.src], m.threshold[base + it.src]};
-                stack.push_back({2 * it.heap + 1, it.d + 1, m.left[base + it.src]});
-                stack.push_back({2 * it.heap + 2, it.d + 1, m.right[base + it.src]});
-              }
-            }
-          }
-          o_nodes[mi] = tb.add(hn);
-          o_leaves[mi] = tb.add(hl);
-          o_slot[mi] = tb.add(m.tree_slot);
-          o_scale[mi] = tb.add(m.tree_scale);
-          t2m[mi].n_trees = nt;
-          t2m[mi].depth = D;
-          t2m[mi].n_internal = ni;
-          t2m[mi].n_leaves = nl;
-        }
-        const size_t o_models2 = align_up(tb.data.size(), 16);
-        tb.data.resize(o_models2 + sizeof(T2Model) * M);
-        CUDA_TRY(cudaMalloc(&p->d_t2_blob, tb.data.size()));
-        for (int mi = 0; mi < M; ++mi) {
-          t2m[mi].nodes = (const HeapNode*)(p->d_t2_blob + o_nodes[mi]);
-          t2m[mi].leaves = (const double*)(p->d_t2_blob + o_leaves[mi]);
-          t2m[mi].slot = (const int32_t*)(p->d_t2_blob + o_slot[mi]);
-          t2m[mi].scale = (const double*)(p->d_t2_blob + o_scale[mi]);
-        }
-        memcpy(tb.data.data() + o_models2, t2m.data(), sizeof(T2Model) * M);
-        CUDA_TRY(cudaMemcpy(p->d_t2_blob, tb.data.data(), tb.data.size(), cudaMemcpyHostToDevice));
-        T2Params& t = p->t2;
-        memset(&t, 0, sizeof(t));
-        t.n_in = n_in;
-        t.n_models = M;
-        t.tile_rows = TR2;
-        t.pitch = pitch;
-        t.stages = ST2;
-        t.groups = G2;
-        t.t2 = (const T2Model*)(p->d_t2_blob + o_models2);
-        t.models = k.models;
-        t.classes = k.classes;
-        t.bias = k.bias;
-        t.sm_tables = 0;
-        t.sm_part = (int)align_up(max_table, 16);
-        t.sm_tiles = (int)(align_up(max_table, 16) + align_up(part_bytes, 16));
-        p->t2_smem = (int)total2;
-        p->t2_NS = NS2;
-        p->t2_block = TR2 * G2;
-        p->t2_grid = std::max(M, (sms / M) * M);
-        p->t2_ok = true;
-        p->kernels_per_batch = 2;
-      }
     }
     for (int i = 0; i < 4; ++i) CUDA_TRY(cudaEventCreate(&p->ev[i]));
     p->finalized = true;
@@ -1890,14 +1535,10 @@ extern "C" int b2s_plan_finalize(b2s_plan_t p) {
 extern "C" const char* b2s_plan_kernel(b2s_plan_t p) {
   if (!p || !p->finalized) return "";
   static thread_local char buf[200];
-  int lm = rt_load_mode();
-  if (lm == 2 && !(p->rt_NCH >= 8 && p->n_in == p->rt_NCH * 4 && tensor_map_encoder())) lm = 1;
+  const bool tmap = rt_tmap_ok(p);
   if (p->dense_ok) snprintf(buf, sizeof(buf), "dense_head_kernel<N=%d> (tcgen05.mma kind::tf32, %s, TMEM accumulator groups; %d scores over %d columns)", p->dense.n_pad, p->dense.exact ? "exact 3-term input split" : "2-term input split", p->dense.n_scores, p->dense.n_in);
-  else if (p->t3_ok) snprintf(buf, sizeof(buf), "t3_prep_kernel + trees3_kernel<D=%d,%s> + t3_vote_kernel (%d parts resident in shared memory, %d walking warps%s)", p->t3_D, p->t3_miss ? "NaN routing" : "floats", p->t3_parts, p->t3.warps, p->t3_top ? ", top levels in the constant bank" : "");
-  else if (p->t2_ok) snprintf(buf, sizeof(buf), "trees_model_kernel<%d> + vote_kernel (models resident in shared memory)", p->t2_NS);
-  else if (p->rt_ok && p->rm_ok && lm == 2) snprintf(buf, sizeof(buf), "rowmma_kernel<NCH=%d,NS=%d> (DMMA m8n8k4 fp64, %d warps x %d stages of 32-row TMA tiles per SM)", p->rt_NCH, p->rt_NS, p->rm_warps, p->rm_stages);
-  else if (p->rt_ok) snprintf(buf, sizeof(buf), "rowthread_kernel<NCH=%d,NS=%d,TPR=%d,RPT=%d,%s>", p->rt_NCH, p->rt_NS, p->rt_TPR, lm == 2 ? p->rt_RPT : 1, lm == 2 ? "TMA tensor-map loads" : (lm == 1 ? "TMA bulk loads" : "cp.async loads"));
-  else if (p->rw_ok) snprintf(buf, sizeof(buf), "rowwarp_kernel<L=%d,CPL=%d,NS=%d,U=%d,CS=%d>", p->rw_L, p->rw_CPL, p->rw_NS, p->rw_U, p->rw_CS);
+  else if (p->t3_ok) snprintf(buf, sizeof(buf), "t3_prep_kernel + trees3_kernel<D=%d,%s> + t3_vote_kernel (%d parts resident in shared memory, %d walking warps)", p->t3_D, p->t3_miss ? "NaN routing" : "floats", p->t3_parts, p->t3.warps);
+  else if (p->rt_ok) snprintf(buf, sizeof(buf), "rowthread_kernel<NCH=%d,NS=%d,TPR=%d,%s>", p->rt_NCH, p->rt_NS, rt_tpr(p->rt_NCH), tmap ? "TMA tensor-map loads" : "TMA bulk loads");
   else snprintf(buf, sizeof(buf), "rows_kernel<%s,NS=%d>", p->mode == MODE_LINEAR ? "LINEAR" : (p->mode == MODE_TREES ? "TREES" : "STORE"), p->NS);
   return buf;
 }
@@ -1922,7 +1563,7 @@ struct NvtxRange {  // one range per plan launch, named after the kernel family 
 static int launch_on(b2s_plan_t p, const void* d_rows, int64_t n_rows, int64_t stride, void* d_out, int32_t* d_status,
                      cudaStream_t st, bool host_rows = false) {
   if (n_rows == 0) return B2S_OK;
-  NvtxRange nvtx(p->dense_ok ? "b2s:dense_head" : p->t3_ok ? "b2s:trees3 (prep+walk+vote)" : p->t2_ok ? "b2s:trees2"
+  NvtxRange nvtx(p->dense_ok ? "b2s:dense_head" : p->t3_ok ? "b2s:trees3 (prep+walk+vote)"
                  : p->rt_ok ? "b2s:rowthread" : p->mode == MODE_STORE ? "b2s:rows_store" : "b2s:rows_kernel");
   KParams k = p->kp;
   k.rows = (const char*)d_rows;
@@ -1961,14 +1602,6 @@ static int launch_on(b2s_plan_t p, const void* d_rows, int64_t n_rows, int64_t s
       k.sig.timeout_ns = fused_timeout_ns;
       c->fused_epoch = k.sig.wait_epoch;
     }
-    // lab switches (profiles/lab/comm_lab.py): which part of a merged step costs what.  Results are NOT merged with them.
-    static const int lab_selfonly = getenv("B2S_LAB_COMM_SELFONLY") ? atoi(getenv("B2S_LAB_COMM_SELFONLY")) : 0;
-    static const int lab_nosignal = getenv("B2S_LAB_COMM_NOSIGNAL") ? atoi(getenv("B2S_LAB_COMM_NOSIGNAL")) : 0;
-    if (lab_selfonly) {
-      k.n_peers = 1;
-      k.peers[0] = (float*)c->buf(c->rank, e);
-    }
-    if (lab_nosignal) k.sig.n = 0;
   }
   if (p->t3_ok) {
     const int C = p->t3_cols;
@@ -1976,7 +1609,7 @@ static int launch_on(b2s_plan_t p, const void* d_rows, int64_t n_rows, int64_t s
     b2s_plan_s::TreeScratch sc;
     {
       std::lock_guard<std::mutex> lk(p->scratch_mu);
-      b2s_plan_s::TreeScratch& mine = p->t2_scratch[st];
+      b2s_plan_s::TreeScratch& mine = p->t3_scratch[st];
       if (n_rows > mine.rows) {  // cudaFree waits for the work that still reads the old buffers
         if (mine.pred) cudaFree(mine.pred);
         if (mine.row_bad) cudaFree(mine.row_bad);
@@ -1999,8 +1632,7 @@ static int launch_on(b2s_plan_t p, const void* d_rows, int64_t n_rows, int64_t s
     pr.vec_ok = k.vec_ok;
     alignas(64) CUtensorMap tmap;
     memset(&tmap, 0, sizeof(tmap));
-    static const int t3_tma = getenv("B2S_T3_TMA") ? atoi(getenv("B2S_T3_TMA")) : 1;
-    pr.use_tmap = (t3_tma && !host_rows && pr.vec_ok && (p->n_in % 32) == 0 && encode_rows_map(&tmap, d_rows, n_rows, stride, p->n_in, kT3TR)) ? 1 : 0;
+    pr.use_tmap = (!host_rows && pr.vec_ok && (p->n_in % 32) == 0 && encode_rows_map(&tmap, d_rows, n_rows, stride, p->n_in, kT3TR)) ? 1 : 0;
     const int resident = std::max(1, (int)G.prop.sharedMemPerMultiprocessor / std::max(p->t3_prep_smem + 1024, 1));
     const int pgrid = (int)std::max<int64_t>(1, std::min<int64_t>(n_tiles, (int64_t)G.prop.multiProcessorCount * std::min(resident, 4)));
     G.launches.fetch_add(3, std::memory_order_relaxed);
@@ -2011,57 +1643,11 @@ static int launch_on(b2s_plan_t p, const void* d_rows, int64_t n_rows, int64_t s
     t.n_rows = n_rows;
     t.partial = sc.pred;
     t.col_stride = sc.rows;
-    e3 = t3_launch_walk(t, p->t3_top.get(), p->t3_D, p->t3_miss, p->t3_grid, p->t3_block, p->t3_smem, (int)G.prop.sharedMemPerBlockOptin, st);
+    e3 = t3_launch_walk(t, p->t3_D, p->t3_miss, p->t3_grid, p->t3_block, p->t3_smem, (int)G.prop.sharedMemPerBlockOptin, st);
     if (e3 != cudaSuccess) return fail(B2S_ERR_CUDA, "tree kernel launch failed: %s", cudaGetErrorString(e3));
     const int vgrid = (int)std::max<int64_t>(1, std::min<int64_t>(4 * G.prop.multiProcessorCount, (n_rows + 255) / 256));
     e3 = t3_launch_vote(k, sc.pred, sc.rows, p->d_t3_col_score, C, sc.row_bad, vgrid, st);
     if (e3 != cudaSuccess) return fail(B2S_ERR_CUDA, "vote kernel launch failed: %s", cudaGetErrorString(e3));
-    return B2S_OK;
-  }
-  if (p->t2_ok) {
-    b2s_plan_s::TreeScratch sc;
-    {
-      std::lock_guard<std::mutex> lk(p->scratch_mu);
-      b2s_plan_s::TreeScratch& mine = p->t2_scratch[st];
-      if (n_rows > mine.rows) {  // cudaFree waits for the work that still reads the old buffers
-        if (mine.pred) { cudaFree(mine.pred); cudaFree(mine.row_bad); }
-        mine = b2s_plan_s::TreeScratch{};
-        const int64_t cap = std::max<int64_t>(n_rows, 65536);
-        CUDA_TRY(cudaMalloc(&mine.pred, (size_t)cap * p->kp.n_models * 8));
-        CUDA_TRY(cudaMalloc(&mine.row_bad, (size_t)cap * 4));
-        mine.rows = cap;
-      }
-      sc = mine;
-    }
-    T2Params t = p->t2;
-    t.rows = (const char*)d_rows;
-    t.row_stride = stride;
-    t.n_rows = n_rows;
-    t.pred = sc.pred;
-    t.row_bad = sc.row_bad;
-    t.vec_ok = k.vec_ok;
-    static std::atomic<bool> t2_attr{false};
-    if (!t2_attr) {
-      CUDA_TRY(cudaFuncSetAttribute(trees_model_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G.prop.sharedMemPerBlockOptin));
-      CUDA_TRY(cudaFuncSetAttribute(trees_model_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G.prop.sharedMemPerBlockOptin));
-      t2_attr = true;
-    }
-    const int64_t tiles2 = (n_rows + t.tile_rows - 1) / t.tile_rows;
-    const int M2 = p->kp.n_models;
-    const int grid2 = (int)std::max<int64_t>(M2, std::min<int64_t>(p->t2_grid, tiles2 * M2));
-    G.launches.fetch_add(2, std::memory_order_relaxed);
-    alignas(64) CUtensorMap tmap;
-    memset(&tmap, 0, sizeof(tmap));
-    static const int t2_tma = getenv("B2S_T2_TMA") ? atoi(getenv("B2S_T2_TMA")) : 1;
-    t.use_tmap = (t2_tma && !host_rows && t.vec_ok && (p->n_in % 32) == 0 && encode_rows_map(&tmap, d_rows, n_rows, stride, p->n_in, t.tile_rows)) ? 1 : 0;
-    if (p->t2_NS == 1) trees_model_kernel<1><<<grid2, p->t2_block, p->t2_smem, st>>>(t, tmap);
-    else trees_model_kernel<4><<<grid2, p->t2_block, p->t2_smem, st>>>(t, tmap);
-    cudaError_t e2 = cudaGetLastError();
-    if (e2 != cudaSuccess) return fail(B2S_ERR_CUDA, "tree kernel launch failed: %s", cudaGetErrorString(e2));
-    const int vgrid = (int)std::max<int64_t>(1, std::min<int64_t>(4 * G.prop.multiProcessorCount, (n_rows + 255) / 256));
-    vote_kernel<<<vgrid, 256, 0, st>>>(k, sc.pred, sc.row_bad);
-    e2 = cudaGetLastError();
-    if (e2 != cudaSuccess) return fail(B2S_ERR_CUDA, "vote kernel launch failed: %s", cudaGetErrorString(e2));
     return B2S_OK;
   }
   if (p->dense_ok && !host_rows && k.vec_ok) {
@@ -2085,22 +1671,6 @@ static int launch_on(b2s_plan_t p, const void* d_rows, int64_t n_rows, int64_t s
     lc.host_rows = host_rows;
     cudaError_t e = rt_launch(p, d_rows, stride, n_rows, d_out, d_status, k.vec_ok, st, false, nullptr, nullptr, &lc);
     if (e != cudaSuccess) return fail(B2S_ERR_CUDA, "row-thread kernel launch failed: %s", cudaGetErrorString(e));
-    return B2S_OK;
-  }
-  if (p->rw_ok && k.vec_ok && k.n_peers == 0 && !p->comm && !host_rows) {
-    RWParams r = p->rw;
-    r.rows = (const char*)d_rows;
-    r.row_stride = stride;
-    r.n_rows = n_rows;
-    r.out = (float*)d_out;
-    r.status = d_status;
-    const int rpw = 32 / p->rw_L;
-    const int u = p->rw_U;
-    const int64_t groups = (n_rows + (int64_t)u * rpw - 1) / ((int64_t)u * rpw);
-    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(p->rw_grid, (groups + 3) / 4));
-    G.launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t e = launch_rw(p->rw_L, p->rw_CPL, p->rw_NS, p->rw_CS, r, grid, p->rw_smem, st);
-    if (e != cudaSuccess) return fail(B2S_ERR_CUDA, "row-warp kernel launch failed: %s", cudaGetErrorString(e));
     return B2S_OK;
   }
   // small batches: shrink the tile so that every SM gets work (latency path); the shared-memory
@@ -2135,7 +1705,7 @@ int b2s_int_launch_gathered(b2s_plan_s* p, const B2SGather& g, long long n, void
   static const int fused = getenv("B2S_ENRICH_FUSED") ? atoi(getenv("B2S_ENRICH_FUSED")) : 1;
   // the gather loader lives in the row-thread kernel (linear models, rows of whole 16-byte chunks); with a table impute
   // policy, one-hot sources would need the policy applied before the category search: those plans gather first
-  if (!fused || !p->rt_ok || p->t2_ok || p->t3_ok || (p->n_in % 4) != 0) return fail(B2S_ERR_UNSUPPORTED, "plan is not fusable with the gather");
+  if (!fused || !p->rt_ok || p->t3_ok || (p->n_in % 4) != 0) return fail(B2S_ERR_UNSUPPORTED, "plan is not fusable with the gather");
   if (g.any_impute && p->rt_cat_cols > 0) return fail(B2S_ERR_UNSUPPORTED, "one-hot columns under a table impute policy gather first");
   if (n <= 0) return B2S_OK;
   G.launches.fetch_add(1, std::memory_order_relaxed);
@@ -2791,9 +2361,8 @@ extern "C" int b2s_plan_destroy(b2s_plan_t p) {
       if (p->ev[i]) cudaEventDestroy(p->ev[i]);
     for (cudaEvent_t e : p->chunk_ev) cudaEventDestroy(e);
     if (p->d_blob) cudaFree(p->d_blob);
-    if (p->d_t2_blob) cudaFree(p->d_t2_blob);
     if (p->d_t3_blob) cudaFree(p->d_t3_blob);
-    for (auto& kv : p->t2_scratch)
+    for (auto& kv : p->t3_scratch)
       if (kv.second.pred) { cudaFree(kv.second.pred); cudaFree(kv.second.row_bad); if (kv.second.xt) cudaFree(kv.second.xt); }
     delete p;
     return B2S_OK;
@@ -2973,27 +2542,8 @@ static int comm_wait_epoch(b2s_comm_t c, void* stream, uint32_t e, const void** 
     uint32_t* timeout_flag = reinterpret_cast<uint32_t*>(c->base) + 65;
     // how long a rank may lag behind before the step is declared dead (B2S_COMM_TIMEOUT_MS, default 10 s)
     static const long long timeout_ns = (getenv("B2S_COMM_TIMEOUT_MS") ? atoll(getenv("B2S_COMM_TIMEOUT_MS")) : 10000ll) * 1000000ll;
-    static const int lab_nowait = getenv("B2S_LAB_COMM_NOWAIT") ? atoi(getenv("B2S_LAB_COMM_NOWAIT")) : 0;  // lab: no wait at all
-    // A one-warp polling kernel (gives up after B2S_COMM_TIMEOUT_MS).  B2S_COMM_WAIT=memop: stream memory operations instead
-    // (cuStreamBatchMemOp, one WAIT_VALUE_32 >= e per source rank; no kernel, no timeout) -- measured SLOWER than the kernel
-    // (0.0641 vs 0.0601 ms per merged step, r2r), kept for A/B runs.  The cheap form is the fused wait (b2s_comm_set_fused_wait).
-    static const bool want_memop = getenv("B2S_COMM_WAIT") && std::string(getenv("B2S_COMM_WAIT")) == "memop";
-    BatchMemOpFn memop = want_memop ? stream_batch_memop() : nullptr;
-    if (lab_nowait) {
-    } else if (memop) {
-      CUstreamBatchMemOpParams ops[8];
-      memset(ops, 0, sizeof(ops));
-      for (int g = 0; g < c->world; ++g) {
-        ops[g].waitValue.operation = CU_STREAM_MEM_OP_WAIT_VALUE_32;
-        ops[g].waitValue.address = (CUdeviceptr)(uintptr_t)(c->flags(c->rank) + g);
-        ops[g].waitValue.value = e;
-        ops[g].waitValue.flags = CU_STREAM_WAIT_VALUE_GEQ;  // (int32)(*addr - e) >= 0: wrap-safe like the kernel's test
-      }
-      const CUresult r = memop((CUstream)st, (unsigned)c->world, ops, 0);
-      if (r != CUDA_SUCCESS) return fail(B2S_ERR_CUDA, "cuStreamBatchMemOp (merge wait) failed: %d", (int)r);
-    } else {
-      merge_wait_kernel<<<1, 32, 0, st>>>(c->flags(c->rank), c->world, e, timeout_flag, timeout_ns);
-    }
+    // A one-warp polling kernel.  The cheap form is the fused wait (b2s_comm_set_fused_wait), which launches nothing.
+    merge_wait_kernel<<<1, 32, 0, st>>>(c->flags(c->rank), c->world, e, timeout_flag, timeout_ns);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(B2S_ERR_CUDA, "merge wait launch failed: %s", cudaGetErrorString(err));
     G.launches.fetch_add(1, std::memory_order_relaxed);

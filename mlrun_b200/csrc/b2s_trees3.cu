@@ -23,44 +23,21 @@ cudaError_t t3_launch_prep(const T3Prep& pr, const CUtensorMap& tmap, bool miss,
   return cudaGetLastError();
 }
 
-template <int D, bool MISS, int U>
+template <int D, bool MISS>
 static cudaError_t walk(const T3Params& t, int grid, int block, int smem, int smem_optin, cudaStream_t st) {
   static std::atomic<bool> attr{false};
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(trees3_kernel<D, MISS, U>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+    cudaError_t e = cudaFuncSetAttribute(trees3_kernel<D, MISS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
     if (e != cudaSuccess) return e;
     attr = true;
   }
-  trees3_kernel<D, MISS, U><<<grid, block, smem, st>>>(t);
+  trees3_kernel<D, MISS><<<grid, block, smem, st>>>(t);
   return cudaGetLastError();
 }
 
-template <int D, bool MISS>
-static cudaError_t walk_top(const T3Params& t, const T3Top& top, int grid, int block, int smem, int smem_optin, cudaStream_t st) {
-  static std::atomic<bool> attr{false};
-  if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(trees3_top_kernel<D, MISS, kT3U>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
-    if (e != cudaSuccess) return e;
-    attr = true;
-  }
-  trees3_top_kernel<D, MISS, kT3U><<<grid, block, smem, st>>>(t, top);
-  return cudaGetLastError();
-}
-
-cudaError_t t3_launch_walk(const T3Params& t, const T3Top* top, int depth, bool miss, int grid, int block, int smem, int smem_optin,
-                           cudaStream_t st) {
-#define B2S_T3_TOP(DD)                                                                                              \
-  if (top && depth == DD)                                                                                           \
-    return miss ? walk_top<DD, true>(t, *top, grid, block, smem, smem_optin, st) : walk_top<DD, false>(t, *top, grid, block, smem, smem_optin, st);
-  B2S_T3_TOP(3) B2S_T3_TOP(4) B2S_T3_TOP(5) B2S_T3_TOP(6) B2S_T3_TOP(7) B2S_T3_TOP(8)
-#undef B2S_T3_TOP
-#define B2S_T3_CASE(DD)                                                                                             \
-  if (depth == DD) {                                                                                                \
-    if (t.unroll > kT3U)                                                                                            \
-      return miss ? walk<DD, true, 2 * kT3U>(t, grid, block, smem, smem_optin, st)                                  \
-                  : walk<DD, false, 2 * kT3U>(t, grid, block, smem, smem_optin, st);                                \
-    return miss ? walk<DD, true, kT3U>(t, grid, block, smem, smem_optin, st) : walk<DD, false, kT3U>(t, grid, block, smem, smem_optin, st); \
-  }
+cudaError_t t3_launch_walk(const T3Params& t, int depth, bool miss, int grid, int block, int smem, int smem_optin, cudaStream_t st) {
+#define B2S_T3_CASE(DD) \
+  if (depth == DD) return miss ? walk<DD, true>(t, grid, block, smem, smem_optin, st) : walk<DD, false>(t, grid, block, smem, smem_optin, st);
   B2S_T3_CASE(2) B2S_T3_CASE(3) B2S_T3_CASE(4) B2S_T3_CASE(5) B2S_T3_CASE(6) B2S_T3_CASE(7) B2S_T3_CASE(8)
 #undef B2S_T3_CASE
   return cudaErrorInvalidValue;

@@ -55,14 +55,6 @@ struct T3Part {           // one per part, in global memory
   int32_t n_cols;         // columns of `partial` this part writes (trees: 1)
   int32_t col0;
   int32_t cta0, n_ctas;   // the CTAs [cta0, cta0 + n_ctas) of the grid work on this part
-  int32_t top0;          // first tree of this part in T3Top (walks that read their top levels from the constant bank)
-};
-
-// The top three levels of every tree (heap nodes 1..7) as a kernel parameter: parameters live in the constant bank, a warp-uniform
-// read from it costs no shared-memory wavefront (the walk's bound).  28 KB of the 32 KB a launch may carry.
-constexpr int kT3TopTrees = 512;
-struct T3Top {
-  uint2 n[kT3TopTrees * 7];
 };
 
 struct T3Prep {           // t3_prep_kernel
@@ -83,18 +75,17 @@ struct T3Params {         // trees3_kernel
   int64_t col_stride;
   const T3Part* parts;
   int32_t n_in, n_parts, warps;  // warps: walking warps (the CTA has kT3Service more)
-  int32_t unroll;                // trees in flight per warp (kT3U or twice that)
   int32_t xt_words;              // words of one tile (n_in rounded up to 4, times TR); two tiles are resident
   int32_t part_words;            // doubles of one partial-sum buffer; two are resident
   int32_t sm_leaf, sm_part, sm_xt, sm_bar;  // byte offsets into dynamic shared memory
   // the linear part: walking warp s < lin_slices takes the feature slice s of every score column; its partial sums live where
   // the tree parts keep their tables (two buffers of lin_part_words doubles at sm_lin_part)
-  int32_t lin_slices, lin_part_words, sm_lin_part, pad0;
+  int32_t lin_slices, lin_part_words, sm_lin_part;
 };
 
 // launchers (b2s_trees3.cu: the kernels are compiled in their own translation unit)
 cudaError_t t3_launch_prep(const T3Prep& pr, const CUtensorMap& tmap, bool miss, int grid, int smem, int smem_optin, cudaStream_t st);
-cudaError_t t3_launch_walk(const T3Params& t, const T3Top* top, int depth, bool miss, int grid, int block, int smem, int smem_optin, cudaStream_t st);
+cudaError_t t3_launch_walk(const T3Params& t, int depth, bool miss, int grid, int block, int smem, int smem_optin, cudaStream_t st);
 cudaError_t t3_launch_vote(const KParams& k, const double* partial, int64_t col_stride, const int32_t* col_score, int n_cols,
                            const int32_t* row_bad, int grid, cudaStream_t st);
 
@@ -263,12 +254,12 @@ __global__ void __launch_bounds__(kT3PrepThreads) t3_prep_kernel(const __grid_co
 }
 
 // ------------------------------------------------------------------------------------------ walk
-template <int D, bool MISS, int U, bool TOPC>
-__device__ __forceinline__ void t3_walk_body(const T3Params& p, const uint2* __restrict__ topn) {
+template <int D, bool MISS>
+__global__ void __launch_bounds__(1024) trees3_kernel(const __grid_constant__ T3Params p) {
   extern __shared__ __align__(1024) unsigned char smem3[];
   unsigned char* const smem = smem3;
   constexpr int NN = 1 << D;  // node slots per tree (1-based heap) == leaves per tree
-  constexpr int TR = kT3TR, RPT = kT3RPT;
+  constexpr int TR = kT3TR, RPT = kT3RPT, U = kT3U;
   const int tid = threadIdx.x, lane = tid & 31, g = tid >> 5;
   const int W = p.warps;                   // walking warps; the last kT3Service warps serve them
   const int n_all = (W + kT3Service) * 32;
@@ -381,56 +372,7 @@ __device__ __forceinline__ void t3_walk_body(const T3Params& p, const uint2* __r
         }
         uint2 nd[U][RPT];
         uint32_t x[U][RPT];
-        if constexpr (TOPC) {  // levels 0..2 from the constant bank: nodes 1..7 of the tree, no shared-memory traffic
-          uint2 n[U][7];
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            const uint2* tp = topn + (size_t)(part.top0 + (valid[u] ? g + (i + u) * W : 0)) * 7;
-#pragma unroll
-            for (int q = 0; q < 7; ++q) n[u][q] = tp[q];
-          }
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            x[u][0] = t3_lds32<0>(xls + t3_xoff<MISS>(n[u][0].x));
-            if (RPT > 1) x[u][1] = t3_lds32<128>(xls + t3_xoff<MISS>(n[u][0].x));
-          }
-          bool r0[U][RPT], r1[U][RPT];
-#pragma unroll
-          for (int u = 0; u < U; ++u)
-#pragma unroll
-            for (int j = 0; j < RPT; ++j) {
-              r0[u][j] = t3_right<MISS>(x[u][j], n[u][0]);
-              nd[u][j].x = r0[u][j] ? n[u][2].x : n[u][1].x;
-              nd[u][j].y = r0[u][j] ? n[u][2].y : n[u][1].y;
-            }
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            x[u][0] = t3_lds32<0>(xls + t3_xoff<MISS>(nd[u][0].x));
-            if (RPT > 1) x[u][1] = t3_lds32<128>(xls + t3_xoff<MISS>(nd[u][1].x));
-          }
-#pragma unroll
-          for (int u = 0; u < U; ++u)
-#pragma unroll
-            for (int j = 0; j < RPT; ++j) {
-              r1[u][j] = t3_right<MISS>(x[u][j], nd[u][j]);
-              const uint32_t lx = r1[u][j] ? n[u][4].x : n[u][3].x, ly = r1[u][j] ? n[u][4].y : n[u][3].y;
-              const uint32_t hx = r1[u][j] ? n[u][6].x : n[u][5].x, hy = r1[u][j] ? n[u][6].y : n[u][5].y;
-              nd[u][j].x = r0[u][j] ? hx : lx;
-              nd[u][j].y = r0[u][j] ? hy : ly;
-            }
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            x[u][0] = t3_lds32<0>(xls + t3_xoff<MISS>(nd[u][0].x));
-            if (RPT > 1) x[u][1] = t3_lds32<128>(xls + t3_xoff<MISS>(nd[u][1].x));
-          }
-#pragma unroll
-          for (int u = 0; u < U; ++u)
-#pragma unroll
-            for (int j = 0; j < RPT; ++j) {
-              const bool r2 = t3_right<MISS>(x[u][j], nd[u][j]);
-              a[u][j] = tba[u] + 64u + (r0[u][j] ? 32u : 0u) + (r1[u][j] ? 16u : 0u) + (r2 ? 8u : 0u);
-            }
-        } else {  // levels 0 and 1: nodes 1..3 of the tree, one warp-uniform LDS.64 + LDS.128 for all RPT row blocks
+        {  // levels 0 and 1: nodes 1..3 of the tree, one warp-uniform LDS.64 + LDS.128 for all RPT row blocks
           uint2 n1[U], n2[U], n3[U];
 #pragma unroll
           for (int u = 0; u < U; ++u) {
@@ -467,7 +409,7 @@ __device__ __forceinline__ void t3_walk_body(const T3Params& p, const uint2* __r
             }
         }
 #pragma unroll
-        for (int d = TOPC ? 3 : 2; d < D; ++d) {
+        for (int d = 2; d < D; ++d) {
 #pragma unroll
           for (int u = 0; u < U; ++u)
 #pragma unroll
@@ -532,15 +474,6 @@ __device__ __forceinline__ void t3_walk_body(const T3Params& p, const uint2* __r
     __syncwarp();
     if (lane == 0) t3_mbar_arrive(&s_done[buf]);  // release: the stores above are visible to whoever completes the wait
   }
-}
-
-template <int D, bool MISS, int U>
-__global__ void __launch_bounds__(1024) trees3_kernel(const __grid_constant__ T3Params p) {
-  t3_walk_body<D, MISS, U, false>(p, nullptr);
-}
-template <int D, bool MISS, int U>
-__global__ void __launch_bounds__(1024) trees3_top_kernel(const __grid_constant__ T3Params p, const __grid_constant__ T3Top top) {
-  t3_walk_body<D, MISS, U, true>(p, top.n);
 }
 
 // Per row: scores = init + the model's columns of `partial` in column order, link, then the VotingEnsemble reduce.

@@ -96,9 +96,9 @@ def test_depths(depth, n_trees):
 
 
 @pytest.mark.parametrize("depth,routes_nan", [(3, False), (6, False), (5, True)])
-def test_top_levels_from_the_constant_bank_equal_the_shared_memory_walk(depth, routes_nan, monkeypatch):
-    """B2S_T3_TOPC=1: the walk reads heap nodes 1..7 of every tree from the launch parameters (constant bank) instead of
-    shared memory (the default; measured equal): same comparisons, same fp64 adds in the same order -> bit-identical outputs"""
+def test_walk_levels_match_the_oracle(depth, routes_nan):
+    """the top two levels of every tree are read with warp-uniform loads, the rest node by node: both against predict(),
+    with and without NaN routing"""
     if routes_nan:
         from sklearn.ensemble import RandomForestRegressor
 
@@ -112,16 +112,23 @@ def test_top_levels_from_the_constant_bank_equal_the_shared_memory_walk(depth, r
     else:
         wl = tree_workload(n_rows=1500, n_feat=16, n_models=2, n_trees=20, depth=depth, seed=60 + depth, n_fit=3000)
         models, X = wl.models, wl.X
-    packed = [packing.pack_model(m) for m in models]
-    monkeypatch.setenv("B2S_T3_TOPC", "1")
-    plan = ColumnProgram(names(16)).build_plan(packed)
-    assert "top levels in the constant bank" in plan.kernel, plan.kernel
-    got = plan.run(X)
-    monkeypatch.delenv("B2S_T3_TOPC")
-    shared = ColumnProgram(names(16)).build_plan(packed)
-    assert "constant bank" not in shared.kernel and "trees3_kernel" in shared.kernel, shared.kernel
-    assert np.array_equal(got, shared.run(X))
-    np.testing.assert_allclose(got, np.stack([m.predict(X.astype(np.float64)) for m in models], axis=1), rtol=RTOL, atol=ATOL)
+    plan = ColumnProgram(names(16)).build_plan([packing.pack_model(m) for m in models])
+    assert f"trees3_kernel<D={depth},{'NaN routing' if routes_nan else 'floats'}>" in plan.kernel, plan.kernel
+    np.testing.assert_allclose(plan.run(X), np.stack([m.predict(X.astype(np.float64)) for m in models], axis=1), rtol=RTOL, atol=ATOL)
+
+
+def test_rows_too_wide_for_the_parts_kernel_take_the_generic_tree_kernel():
+    """432 columns: two transposed 64-row tiles fill a CTA's shared memory, so no part fits next to them and the plan runs on
+    the generic rows_kernel<TREES>"""
+    wl = tree_workload(n_rows=3000, n_feat=432, n_models=4, n_trees=10, depth=2, seed=12, n_fit=600)
+    packed = [packing.pack_model(m) for m in wl.models]
+    ref = obatch.tree_ensemble(wl)
+    plan = ColumnProgram(names(432)).build_plan(packed, vote=(nat.VOTE_MEAN, [0.25] * 4))
+    assert plan.kernel.startswith("rows_kernel<TREES"), plan.kernel
+    out, status = plan.run(wl.X, with_status=True)
+    np.testing.assert_allclose(out[:, 0], ref["out"], rtol=RTOL, atol=ATOL)
+    assert not status.any()
+    np.testing.assert_allclose(ColumnProgram(names(432)).build_plan(packed).run(wl.X), ref["per_model"], rtol=RTOL, atol=ATOL)
 
 
 def test_a_model_larger_than_one_cta_is_split_into_parts():
